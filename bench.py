@@ -2,10 +2,12 @@
 """bench.py -- the reference's headline metric (BASELINE.json) on B200:
 "NTT Melem/s at 2^20; LDE+Merkle-commit ms/proof at 1/2/4/8 B200".
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
-One JSON line (rank 0).  What is in it:
+One JSON line (rank 0).  `--dump-outputs DIR` also writes rank 0's output of the last timed step
+(a fixed, seeded sample of its points; see dump_outputs) to DIR, so that two builds can be compared
+output for output: the inputs are seeded and the same in every run.  What is in the line:
 
   value / ms_per_step   forward NTT of `--cols` (64) columns x 2^20 per GPU, inputs resident in
                         HBM (2 GiB in, 2 GiB out: larger than L2), CUDA events on the launching
@@ -211,6 +213,24 @@ def synth_columns(cols, n, seed):
   a = rng.integers(0, 2**32, size=(cols, n, 8), dtype=np.uint64).astype(np.uint32)
   a[:, :, 7] &= 0x7FFFFFFF  # < 2^255 < p: canonical residues
   return a
+
+
+DUMP_POINTS = 8192     # sampled points per column: 64 columns x 8192 x 8 limbs in float64 = 32 MiB
+DUMP_SEED = 20        # fixed: every run and every build samples the same points
+
+
+def dump_outputs(out_dir, torch, d_out):
+  """Writes what the timed NTT handed back in its last step to out_dir as .npy files:
+  ntt_out_limbs.npy (cols, DUMP_POINTS, 8): the eight little-endian 32-bit limbs of every column at
+  a fixed, seeded sample of evaluation points, as float64 (exact for 32-bit values);
+  ntt_out_points.npy (DUMP_POINTS,): the sampled point indices."""
+  import numpy as np
+  cols, n, _ = d_out.shape
+  pts = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(DUMP_POINTS, n), replace=False))
+  limbs = d_out[:, torch.from_numpy(pts).to(d_out.device), :].cpu().numpy().view(np.uint32)
+  os.makedirs(out_dir, exist_ok=True)
+  np.save(os.path.join(out_dir, "ntt_out_limbs.npy"), limbs.astype(np.float64))
+  np.save(os.path.join(out_dir, "ntt_out_points.npy"), pts.astype(np.float64))
 
 
 def numa_note():
@@ -746,7 +766,13 @@ def main():
   ap.add_argument("--no-e2e", action="store_true")
   ap.add_argument("--no-extras", action="store_true", help="skip configs 3, 4, 5 (LDE+commit, 2^26 NTT, full proof)")
   ap.add_argument("--no-pyref", action="store_true", help="skip the pure-Python reference timings (~80 s)")
+  ap.add_argument("--dump-outputs", metavar="DIR",
+                  help="write a fixed sample of the last timed step's NTT output to DIR/*.npy (rank 0)")
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
+  if args.dump_outputs and args.impl == "reference":
+    ap.error("--dump-outputs applies to the GPU implementation only")
   rank = int(os.environ.get("RANK", "0"))
   world = int(os.environ.get("WORLD_SIZE", "1"))
   local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -801,6 +827,8 @@ def main():
   barrier()
   ms = e0.elapsed_time(e1)
   clocks = sampler.stop()
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, torch, d_out)
   # e2e through the host-buffer API
   e2e_s, pcie_duplex = None, None
   if not args.no_e2e:

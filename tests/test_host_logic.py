@@ -2,7 +2,6 @@
 Fiat-Shamir helpers, Merkle index arithmetic and the verifier -- exercised on proofs made by
 the CPU oracle."""
 import hashlib
-import os
 
 import numpy as np
 import pytest
@@ -115,23 +114,62 @@ def test_verifier_accepts_oracle_proofs_and_rejects_tampering(oracle):
     FRI(F).verify_proximity_proof(prf, b"\1" * 32, F(w), deg, exclude_multiples_of=8)
 
 
-def test_install_rebinds_reference_when_present():
+# A stand-in for the upstream `starks` package: the module attributes install() replaces, `from x
+# import y` aliases of them in starks.fri and starks.stark (as in stark.py:4-17, fri.py:6-8,17), and
+# the FRI class present as oracle/pyref.py restores it.  Bodies are irrelevant: nothing is called.
+_UPSTREAM_STAND_IN = {
+    "__init__": "",
+    "fft": ("def fft_1d(field, vals, modulus, root_of_unity, inv=False): raise NotImplementedError\n"
+            "def mul_polys(a, b, root_of_unity): raise NotImplementedError\n"
+            "class NonBinaryFFT(object): pass\n"),
+    "merkle_tree": ("def merkelize(L): raise NotImplementedError\n"
+                    "def merkelize_polynomial_evaluations(dims, polynomial_evals): raise NotImplementedError\n"),
+    "utils": "def get_power_cycle(r, field): raise NotImplementedError\n",
+    "fri": ("from starks.merkle_tree import merkelize\n"
+            "class SmoothSubgroupFRI(object): pass\n"
+            "FRI = SmoothSubgroupFRI\n"),
+    "stark": ("from starks.merkle_tree import merkelize\n"
+              "from starks.fri import FRI\n"
+              "from starks.utils import get_power_cycle\n"
+              "class STARK(object):\n"
+              "  def mk_proof(self, witness, boundary): raise NotImplementedError\n"),
+}
+
+
+def test_install_rebinds_reference_when_present(tmp_path, monkeypatch):
+  """install() rebinds the upstream hot-path names and their aliases; uninstall() puts every one
+  back.  Runs on a stand-in package with the upstream module surface (the upstream source is not
+  part of this repository), so it needs neither the reference tree nor a GPU."""
   import sys
-  sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle"))
-  import pyref
-  if not pyref.available():
-    pytest.skip("upstream reference tree not present")
-  pyref.load()
+  pkg = tmp_path / "starks"
+  pkg.mkdir()
+  for name, src in _UPSTREAM_STAND_IN.items():
+    (pkg / (name + ".py")).write_text(src)
+  for m in [m for m in sys.modules if m == "starks" or m.startswith("starks.")]:
+    monkeypatch.delitem(sys.modules, m)     # a reference loaded by another test comes back afterwards
+  monkeypatch.syspath_prepend(str(tmp_path))
+  try:
+    _install_rebinds_and_restores()
+  finally:
+    for m in [m for m in sys.modules if m == "starks" or m.startswith("starks.")]:
+      del sys.modules[m]
+
+
+def _install_rebinds_and_restores():
+  import sys
   import starks.stark, starks.fft, starks.merkle_tree, starks.fri
   before = {m: dict(vars(sys.modules[m])) for m in ("starks.fft", "starks.merkle_tree", "starks.fri", "starks.stark", "starks.utils")}
   saved_mk = starks.stark.STARK.mk_proof
   import starks_b200.install as shim
   import starks_b200.fft as bfft, starks_b200.merkle_tree as bmt, starks_b200.fri as bfri
+  import starks_b200.utils as butils
   try:
     assert shim.install()
     assert starks.fft.fft_1d is bfft.fft_1d and starks.merkle_tree.merkelize is bmt.merkelize
     assert starks.stark.merkelize is bmt.merkelize and starks.stark.FRI is bfri.FRI
     assert starks.fri.merkelize is bmt.merkelize and starks.fri.SmoothSubgroupFRI is bfri.SmoothSubgroupFRI
+    assert starks.utils.get_power_cycle is butils.get_power_cycle
+    assert starks.stark.get_power_cycle is butils.get_power_cycle
     assert starks.stark.STARK.mk_proof is not saved_mk
     # function-level mode: the upstream prover body stays, only its callees are rebound
     assert shim.install(replace_prover=False)
