@@ -101,16 +101,9 @@ struct stk_peer_leaf {
 };
 int stk_ntt_dev_peer(stk_ctx* c, const stk::fe* d_in, uint64_t n_in, uint64_t in_stride, uint64_t n, uint64_t batch,
                      const stk::fe& root, const stk_peer_leaf& peer);
-// forward transform whose final pass also writes the Merkle bottom level (nodes [n/2, n)) of the
-// column-leaf tree over its `batch` output columns; check eligibility first
-bool stk_ntt_can_fuse_hash(stk_ctx* c, uint64_t n, uint64_t batch);
-int stk_ntt_dev_hash(stk_ctx* c, const stk::fe* d_in, uint64_t n_in, uint64_t in_stride, stk::fe* d_out,
-                     uint64_t out_stride, uint64_t n, uint64_t batch, const stk::fe& root, uint32_t* d_nodes);
 // branch gather with the query indices already on the device; asynchronous (merkle.cu)
 int stk_merkle_paths_dev(stk_ctx* c, const stk::fe* d_cols, uint64_t n, uint64_t ncols, uint64_t col_stride,
                          const uint8_t* d_nodes, const uint64_t* d_idx, uint64_t k, uint32_t* d_out, uint64_t rec_bytes);
-// levels above the bottom one + root download (merkle.cu)
-int stk_merkle_finish(stk_ctx* c, uint8_t* d_nodes, uint64_t np, uint8_t* h_root);
 int stk_ntt_dev(stk_ctx* c, const stk::fe* d_in, uint64_t n_in, uint64_t in_stride, stk::fe* d_out,
                 uint64_t out_stride, uint64_t n, uint64_t batch, const stk::fe& root, int inverse, int scale);
 int stk_ntt_dev_r0(stk_ctx* c, const stk::fe* d_in, uint64_t n_in, uint64_t in_stride, stk::fe* d_out,

@@ -44,20 +44,8 @@ STK_API int stk_lde_commit(stk_ctx* c, const uint32_t* d_trace, uint64_t steps, 
                            uint64_t cols, const uint32_t g2[8], uint32_t* d_evals, uint64_t eval_stride,
                            uint8_t* d_nodes, uint8_t* h_root) {
   if (!c || !d_trace || !d_evals || !d_nodes || !g2 || steps == 0 || ext == 0 || cols == 0) return STK_EINVAL;
-  const uint64_t n = steps * ext;
-  if (stk_ntt_can_fuse_hash(c, n, cols)) {
-    // the forward transform's final pass hashes the leaf pairs itself (ntt.cuh, HASH)
-    fe G2 = stk_load_fe(g2);
-    fe G1 = stk_h_pow(c, G2, ext);
-    void* t;
-    STK_TRY(stk_scratch(c, 1, cols * steps * sizeof(fe), &t));
-    fe* coef = (fe*)t;
-    STK_TRY(stk_ntt_dev(c, (const fe*)d_trace, steps, trace_stride, coef, steps, steps, cols, G1, 1, 1));
-    STK_TRY(stk_ntt_dev_hash(c, coef, steps, steps, (fe*)d_evals, eval_stride, n, cols, G2, (uint32_t*)d_nodes));
-    return stk_merkle_finish(c, d_nodes, n, h_root);
-  }
   STK_TRY(stk_lde(c, d_trace, steps, trace_stride, ext, cols, g2, nullptr, 0, d_evals, eval_stride));
-  return stk_merkle_commit(c, d_evals, n, cols, eval_stride, d_nodes, h_root);
+  return stk_merkle_commit(c, d_evals, steps * ext, cols, eval_stride, d_nodes, h_root);
 }
 
 // stk_lde whose final NTT pass stores every evaluation row directly into the rank that owns

@@ -241,16 +241,6 @@ int reduce_levels(stk_ctx* c, uint32_t* nodes, uint64_t np) {
 
 #define STK_API extern "C" __attribute__((visibility("default")))
 
-int stk_merkle_finish(stk_ctx* c, uint8_t* d_nodes, uint64_t np, uint8_t* h_root) {
-  STK_CUDA(c, cudaMemsetAsync(d_nodes, 0, 32, c->stream));
-  STK_TRY(reduce_levels(c, (uint32_t*)d_nodes, np));
-  if (h_root) {
-    STK_CUDA(c, cudaMemcpyAsync(h_root, d_nodes + 32, 32, cudaMemcpyDeviceToHost, c->stream));
-    STK_CUDA(c, cudaStreamSynchronize(c->stream));
-  }
-  return STK_OK;
-}
-
 int stk_merkle_paths_dev(stk_ctx* c, const fe* d_cols, uint64_t n, uint64_t ncols, uint64_t col_stride,
                          const uint8_t* d_nodes, const uint64_t* d_idx, uint64_t k, uint32_t* d_out, uint64_t rec_bytes) {
   if (!k) return STK_OK;

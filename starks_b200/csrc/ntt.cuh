@@ -19,7 +19,8 @@
 // Butterfly at level with half-size H:  (a, b) -> (a + b, (a - b) * w^((J mod H) * N/(2H))).
 // Twiddles come from one table W[e] = w^e (e < N) kept in HBM in "twiddle form".
 #pragma once
-#include "blake2s.cuh"
+#include <algorithm>
+#include "ctx.h"
 #include "field.cuh"
 
 namespace stk {
@@ -79,14 +80,6 @@ struct NttPass {
   int peer_g;
   uint32_t peer_col0;
   int in_rot;
-  // fused Merkle bottom level (HASH instantiation, final pass of stk_lde_commit): the grid runs
-  // column-fastest (grid_swap), every CTA bumps its tile's counter after its stores, and the CTA
-  // that completes a tile -- all `batch` columns of those rows are now written -- hashes the
-  // tile's leaf pairs straight out of L2 into hash_nodes (heap order, 8 words per node).
-  int hash_on;
-  int grid_swap;
-  uint32_t* hash_nodes;
-  unsigned int* hash_cnt;
   fe* peer_out[8];
   const fe* in;
   fe* out;
@@ -216,68 +209,12 @@ __device__ __forceinline__ void ntt_round(const NttPass& A, const F& f, uint32_t
   }
 }
 
-// Bottom Merkle level of one final-pass tile (merkelize_polynomial_evaluations + the deepest
-// level of merkelize, starks/merkle_tree.py:36-56, 94-119).  The tile holds output rows
-// K = (jr << (n-k)) | (bitrev(tile) << logC) | cr for every jr < 2^k, i.e. whole permute4 quads
-// {u, u+q, u+2q, u+3q} (q = N/4): leaf pair s of quad u is rows (2s*q + u, 2s*q + u + q) and its
-// parent is node N/2 + 2u + s.  Values were stored by other CTAs: read through L2 (ld.cg).
-struct HashTile {  // by value: a reference to the kernel's NttPass would force a local copy of it
-  const fe* out;
-  unsigned long long out_col_stride;
-  uint32_t* nodes;
-  uint32_t ncols;
-  int n, k, logC, logT, nl;
-};
-static __device__ __noinline__ void hash_tile_rows(const HashTile A, uint32_t xb) {
-  const uint32_t T = 1u << A.logT;
-  const uint32_t tr = A.nl ? (__brev(xb) >> (32 - A.nl)) : 0u;
-  const uint32_t Cm = (1u << A.logC) - 1u;
-  const unsigned long long q = 1ull << (A.n - 2), half = 1ull << (A.n - 1);
-  const uint32_t ncols = A.ncols;
-  for (uint32_t p = threadIdx.x; p < (T >> 1); p += blockDim.x) {
-    const uint32_t cr = p & Cm, s = (p >> A.logC) & 1u, jr = p >> (A.logC + 1);
-    const unsigned long long u = ((unsigned long long)jr << (A.n - A.k)) | (tr << A.logC) | cr;
-    const unsigned long long x0 = 2ull * s * q + u, x1 = x0 + q;
-    uint32_t h[8];
-    b2s_init(h);
-    // value v of the pair's 2*ncols-value message: columns of row x0, then columns of row x1
-    auto value_ptr = [&](uint32_t v) {
-      return reinterpret_cast<const uint4*>((v < ncols) ? (A.out + (unsigned long long)v * A.out_col_stride + x0)
-                                                        : (A.out + (unsigned long long)(v - ncols) * A.out_col_stride + x1));
-    };
-    uint4 nx[4];  // the next block's two values are in flight while this block is compressed
-    nx[0] = __ldcg(value_ptr(0)); nx[1] = __ldcg(value_ptr(0) + 1);
-    nx[2] = __ldcg(value_ptr(1)); nx[3] = __ldcg(value_ptr(1) + 1);
-    for (uint32_t b = 0; b < ncols; ++b) {
-      uint32_t m[16];
-#pragma unroll
-      for (int hb = 0; hb < 2; ++hb) {
-        const uint4 lo = nx[2 * hb], hi = nx[2 * hb + 1];
-        m[8 * hb + 0] = bswap32(hi.w); m[8 * hb + 1] = bswap32(hi.z);
-        m[8 * hb + 2] = bswap32(hi.y); m[8 * hb + 3] = bswap32(hi.x);
-        m[8 * hb + 4] = bswap32(lo.w); m[8 * hb + 5] = bswap32(lo.z);
-        m[8 * hb + 6] = bswap32(lo.y); m[8 * hb + 7] = bswap32(lo.x);
-      }
-      if (b + 1 < ncols) {
-        nx[0] = __ldcg(value_ptr(2 * b + 2)); nx[1] = __ldcg(value_ptr(2 * b + 2) + 1);
-        nx[2] = __ldcg(value_ptr(2 * b + 3)); nx[3] = __ldcg(value_ptr(2 * b + 3) + 1);
-      }
-      b2s_compress(h, m, 64u * (b + 1), b + 1 == ncols);
-    }
-    uint4* dst = reinterpret_cast<uint4*>(A.nodes + 8 * (half + 2 * u + s));
-    dst[0] = make_uint4(h[0], h[1], h[2], h[3]);
-    dst[1] = make_uint4(h[4], h[5], h[6], h[7]);
-  }
-}
-
-template <class F, int MAXR, int MAXT = (4096 >> MAXR), int MINB = 1, int ZS = 0, bool HASH = false>
+template <class F, int MAXR, int MAXT = (4096 >> MAXR), int MINB = 1, int ZS = 0>
 __global__ void __launch_bounds__(MAXT, MINB) ntt_pass_kernel(const NttPass A, const F f) {
   extern __shared__ __align__(16) uint32_t sm[];
   const uint32_t T = 1u << A.logT;
   // single-pass transforms put the column groups on grid.x (no 65535 limit), tiles otherwise
-  // (HASH: columns on grid.x so that the CTAs of one tile are dispatched together)
-  const uint32_t bx = (HASH && A.grid_swap) ? blockIdx.y : blockIdx.x;
-  const uint32_t by = (HASH && A.grid_swap) ? blockIdx.x : blockIdx.y;
+  const uint32_t bx = blockIdx.x, by = blockIdx.y;
   const uint32_t xb = A.c_is_col ? 0u : bx;
   const uint32_t Jcta = ((xb & ((1u << A.nl) - 1u)) << A.sl) | ((xb >> A.nl) << A.sh);
   const uint32_t col0 = A.c_is_col ? (bx << A.logC) : by;
@@ -295,21 +232,6 @@ __global__ void __launch_bounds__(MAXT, MINB) ntt_pass_kernel(const NttPass A, c
     else if (r == 2) ntt_round<F, 2, ZS, false>(A, f, sm, T, Jcta, col0, a, first, last);
     else ntt_round<F, 1, ZS, false>(A, f, sm, T, Jcta, col0, a, first, last);
     if (!last) __syncthreads();
-  }
-  if (HASH && A.hash_on) {
-    __shared__ uint32_t s_last;
-    __threadfence();  // this CTA's evaluation rows are visible device-wide before the count
-    __syncthreads();
-    if (threadIdx.x == 0) s_last = atomicAdd(A.hash_cnt + xb, 1u) == A.batch - 1u;
-    __syncthreads();
-    if (s_last) {
-      __threadfence();
-      HashTile H;
-      H.out = A.out; H.out_col_stride = A.out_col_stride; H.nodes = A.hash_nodes; H.ncols = A.batch;
-      H.n = A.n; H.k = A.k; H.logC = A.logC; H.logT = A.logT; H.nl = A.nl;
-      hash_tile_rows(H, xb);
-    }
-    return;
   }
   if (A.peer_on == 2) {
     // Fused leaf exchange of the sharded commit: rows leave for their leaf owners, consecutive
@@ -348,6 +270,30 @@ __global__ void __launch_bounds__(MAXT, MINB) ntt_pass_kernel(const NttPass A, c
       reinterpret_cast<uint4*>(pd + ((A.peer_self << A.peer_log_chunk) | (J & cmask)))[h] = v;
     }
   }
+}
+
+// Host-side launcher of one ntt_pass_kernel instantiation, whose tiles hold up to (1 << MAXR) * MAXT
+// elements.  Each ntt_pass_*.cu instantiates one so that nvcc compiles the heavy kernels in parallel.
+template <class F, int MAXR, int MAXT, int MINB, int ZS>
+static int launch_pass_r(stk_ctx* c, cudaStream_t s, const NttPass& P, const F& f) {
+  static bool attr_done[64] = {};  // cudaFuncSetAttribute is per device
+  if (!attr_done[c->device & 63]) {
+    STK_CUDA(c, cudaFuncSetAttribute(ntt_pass_kernel<F, MAXR, MAXT, MINB, ZS>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, 32 * (1 << MAXR) * MAXT));
+    attr_done[c->device & 63] = true;
+  }
+  const uint32_t T = 1u << P.logT;
+  if (T > (1u << MAXR) * MAXT) return stk_fail(c, STK_EUNSUPPORTED, "tile larger than this instantiation");
+  unsigned threads = std::max(1u, T >> MAXR);
+  uint64_t tiles = P.c_is_col ? 1 : ((1ull << P.n) >> P.logT);
+  uint64_t cols = P.c_is_col ? ((P.batch + (1u << P.logC) - 1) >> P.logC) : P.batch;
+  if (!P.c_is_col && cols > 65535) return stk_fail(c, STK_EUNSUPPORTED, "more than 65535 columns of a multi-pass transform");
+  if (cols > 0x7fffffffull) return stk_fail(c, STK_EUNSUPPORTED, "batch too large");
+  dim3 grid(P.c_is_col ? (unsigned)cols : (unsigned)tiles, P.c_is_col ? 1u : (unsigned)cols);
+  size_t smem = (P.nrounds > 1 || P.peer_on) ? (size_t)32 * T : 0;
+  ntt_pass_kernel<F, MAXR, MAXT, MINB, ZS><<<grid, threads, smem, s>>>(P, f);
+  STK_CUDA(c, cudaGetLastError());
+  return STK_OK;
 }
 
 // W[m + i] = W[i] * wm  for i < m  (table doubling; both operands in twiddle form)

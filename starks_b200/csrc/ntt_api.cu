@@ -246,15 +246,15 @@ int stk_get_table_strided(stk_ctx* c, const fe& root, uint64_t n, const fe** d_t
 
 static int ilog2_u64(uint64_t x) { int l = 0; while ((1ull << l) < x) ++l; return l; }
 
-static int ntt_max_radix() { return 3; }  // radix-4 measured no faster: profiles/r01_ntt_radix_sweep.txt
+// log2 radix of the STARK-prime rounds; radix-4 measured no faster: profiles/r01_ntt_radix_sweep.txt
+static const int kStarkRadix = 3;
 
 // Rounds of a pass.  Where the remainder round (k mod R levels) goes was measured
-// (tools/gpu_knobs.py, profiles/r01_ntt_round_order.txt): last in non-final passes and in
-// 1024-element final passes, first in 2048-element final passes; the spread is 1-3 %.
+// (profiles/r01_ntt_round_order.txt): last in non-final passes and in 1024-element final
+// passes, first in 2048-element final passes; the spread is 1-3 %.
 static void fill_rounds(NttPass& P, int R) {
   int k = P.k, rem = k % R, full = k / R, idx = 0;
-  int pos = P.final_pass ? env_int("STK_NTT_REMPOS_FINAL", P.logT > 10 ? 0 : 9) : env_int("STK_NTT_REMPOS", 9);
-  if (pos > full) pos = full;
+  const int pos = (P.final_pass && P.logT > 10) ? 0 : full;
   for (int i = 0; i <= full; ++i) {
     if (i == pos && rem) P.r[idx++] = rem;
     if (i < full) P.r[idx++] = R;
@@ -266,10 +266,9 @@ static void fill_rounds(NttPass& P, int R) {
 static int build_plan(int n, uint64_t batch, std::vector<NttPass>& plan, int rmax) {
   // 1024-element tiles (4 CTAs/SM) unless 2048-element tiles (2 CTAs/SM) save a whole pass
   // over HBM (n = 11, 21, 22): profiles/r01_ntt_plan_sweep2.txt.  Run-time moduli: 1024 only.
-  int want = ((n + 10) / 11 < (n + 9) / 10) ? 11 : 10;
-  if (rmax < 3) want = 10;
-  const int logT = std::min(want, std::max(6, env_int("STK_NTT_LOGT", want)));
-  const int kmax = std::min(logT, std::max(3, env_int("STK_NTT_KMAX", 11)));
+  int logT = ((n + 10) / 11 < (n + 9) / 10) ? 11 : 10;
+  if (rmax < 3) logT = 10;
+  const int kmax = logT;  // butterfly levels per pass: at most one whole tile
   plan.clear();
   if (n <= kmax) {
     NttPass P;
@@ -310,8 +309,8 @@ static int build_plan(int n, uint64_t batch, std::vector<NttPass>& plan, int rma
   return STK_OK;
 }
 
-// The pass kernels are instantiated in their own translation units (ntt_pass_*.cu) so that
-// they compile in parallel; this file only sees the host-side launchers.
+// The pass kernel and its launcher (ntt.cuh) are instantiated in their own translation units
+// (ntt_pass_*.cu) so that they compile in parallel; this file only sees the launchers.
 int stk_launch_pass_stark(stk_ctx* c, cudaStream_t s, const NttPass& P);      // radix-8 rounds
 int stk_launch_pass_stark_zs(stk_ctx* c, cudaStream_t s, const NttPass& P);   // + zero-skip levels
 int stk_launch_pass_stark_t11(stk_ctx* c, cudaStream_t s, const NttPass& P);     // 2048-element tiles
@@ -319,12 +318,10 @@ int stk_launch_pass_stark_t11_zs(stk_ctx* c, cudaStream_t s, const NttPass& P);
 int stk_launch_pass_stark_cf(stk_ctx* c, cudaStream_t s, const NttPass& P);      // coset transform, final pass
 int stk_launch_pass_stark_t11_cf(stk_ctx* c, cudaStream_t s, const NttPass& P);
 int stk_launch_pass_mont(stk_ctx* c, cudaStream_t s, const NttPass& P);       // run-time modulus, radix-4
-int stk_launch_pass_stark_hash(stk_ctx* c, cudaStream_t s, const NttPass& P);  // final pass + Merkle bottom level
 
 template <class F>
 static int launch_pass(stk_ctx* c, cudaStream_t s, const NttPass& P, const F&) {
   if constexpr (F::kMontgomery) return stk_launch_pass_mont(c, s, P);
-  else if (P.hash_on) return stk_launch_pass_stark_hash(c, s, P);
   else {
   const bool zs = P.zbit < 32 || (P.cshift && !P.in_virtual);  // expansion round / coset scaling on load
   const bool cf = !zs && P.cshift && (P.final_pass || P.cskip0);  // interleaved store / skipped r = 0 columns
@@ -366,19 +363,19 @@ __global__ void r0_copy_kernel(const fe* __restrict__ r0, uint64_t r0_stride, fe
 
 static int ntt_dev_on(stk_ctx* c, cudaStream_t s, int scratch_slot, const fe* d_in, uint64_t n_in, uint64_t in_stride,
                       fe* d_out, uint64_t out_stride, uint64_t n, uint64_t batch, const fe& root, int inverse,
-                      int scale, const stk_peer_leaf* peer = nullptr, uint32_t* hash_nodes = nullptr,
-                      const fe* r0 = nullptr, uint64_t r0_stride = 0) {
+                      int scale, const stk_peer_leaf* peer = nullptr, const fe* r0 = nullptr,
+                      uint64_t r0_stride = 0) {
   if (n == 0 || batch == 0) return STK_OK;
   if (n_in > n) return stk_fail(c, STK_EINDEX, "input length %llu exceeds the order %llu of the root",
                                 (unsigned long long)n_in, (unsigned long long)n);
   if (n > (1ull << 30)) return stk_fail(c, STK_EUNSUPPORTED, "transform length above 2^30");
   // multi-pass launches put the column index in gridDim.y (<= 65535): wider batches run as
   // consecutive column groups on the same stream (the scratch buffer is reused in stream order)
-  if (batch > 32768 && n > 2048 && !peer && !hash_nodes) {
+  if (batch > 32768 && n > 2048 && !peer) {
     for (uint64_t b0 = 0; b0 < batch; b0 += 32768) {
       const uint64_t nb = std::min<uint64_t>(32768, batch - b0);
       STK_TRY(ntt_dev_on(c, s, scratch_slot, d_in + b0 * in_stride, n_in, in_stride, d_out + b0 * out_stride,
-                         out_stride, n, nb, root, inverse, scale, nullptr, nullptr, r0 ? r0 + b0 * r0_stride : nullptr,
+                         out_stride, n, nb, root, inverse, scale, nullptr, r0 ? r0 + b0 * r0_stride : nullptr,
                          r0_stride));
     }
     return STK_OK;
@@ -449,13 +446,13 @@ static int ntt_dev_on(stk_ctx* c, cudaStream_t s, int scratch_slot, const fe* d_
   // Zero-padded forward transform (LDE, n_in <= N/8): eight coset transforms of order N/8 over
   // <w^8> as 8*batch virtual columns (ntt.cuh, cshift) -- the sub-transform's passes split its
   // own bits evenly (2^18: 9+9, 2^20: 10+10) instead of the long transform's (11+10, 8+8+7).
-  if (c->is_stark && !inverse && !peer && !hash_nodes && n_in > 0 && n_in * 8 <= n && logn >= 6 &&
+  if (c->is_stark && !inverse && !peer && n_in > 0 && n_in * 8 <= n && logn >= 6 &&
       (const void*)d_in != (const void*)d_out && env_int("STK_LDE_COSET", 1)) {
     const int logns = logn - 3;
     const uint64_t ns = n >> 3, vb = batch * 8;
-    STK_TRY(build_plan(logns, vb, plan, ntt_max_radix()));
+    STK_TRY(build_plan(logns, vb, plan, kStarkRadix));
     std::vector<NttPass> whole;
-    STK_TRY(build_plan(logn, batch, whole, ntt_max_radix()));
+    STK_TRY(build_plan(logn, batch, whole, kStarkRadix));
     // only where it saves a pass over HBM (N >= 2^23): at equal pass counts the two routes time the
     // same on one GPU (2^21: 17.87 ms both) and the coset route measured slower inside the NCCL
     // sharded commit (profiles/r01b_dist_2gpu.txt), so the long transform keeps the expansion round
@@ -494,12 +491,10 @@ static int ntt_dev_on(stk_ctx* c, cudaStream_t s, int scratch_slot, const fe* d_
       return STK_OK;
     }
   }
-  STK_TRY(build_plan(logn, batch, plan, c->is_stark ? ntt_max_radix() : 2));
+  STK_TRY(build_plan(logn, batch, plan, c->is_stark ? kStarkRadix : 2));
   fe* tmp = nullptr;
   if (peer && (plan.size() < 2 || logn - 2 - peer->g < plan.back().logC))
     return stk_fail(c, STK_EUNSUPPORTED, "peer scatter needs a multi-pass transform (N >= 2^11) and N/4G >= tile width");
-  if (hash_nodes && !stk_ntt_can_fuse_hash(c, n, batch))
-    return stk_fail(c, STK_EUNSUPPORTED, "fused leaf hash: transform shape not eligible");
   bool need_tmp = plan.size() > 1 || (const void*)d_in == (const void*)d_out;
   if (need_tmp) {
     void* t;
@@ -514,7 +509,7 @@ static int ntt_dev_on(stk_ctx* c, cudaStream_t s, int scratch_slot, const fe* d_
     P.do_scale = (P.final_pass && do_scale) ? 1 : 0;
     P.scale = scale_tw;
     P.zbit = 32;
-    if (i == 0 && n_in > 0 && n_in * 8 <= n && P.k >= 3 && c->is_stark && env_int("STK_NTT_ZSKIP", 1)) {
+    if (i == 0 && n_in > 0 && n_in * 8 <= n && P.k >= 3 && c->is_stark) {
       // the top three levels only scale-and-copy: run them as the first (radix-8) round
       P.zbit = ilog2_u64(n_in);             // 2^zbit >= n_in, and 2^zbit <= N/8
       if (P.r[0] != 3) {                    // remainder round goes last in this pass
@@ -547,37 +542,11 @@ static int ntt_dev_on(stk_ctx* c, cudaStream_t s, int scratch_slot, const fe* d_
         P.peer_on = 2; P.peer_g = peer->g; P.peer_col0 = peer->col0;
         for (int r2 = 0; r2 < (1 << peer->g); ++r2) P.peer_out[r2] = (fe*)(uintptr_t)peer->ptrs[r2];
       }
-      if (hash_nodes) {  // one counter per tile, zeroed in stream order before the pass
-        const uint64_t tiles = n >> P.logT;
-        void* cnt;
-        STK_TRY(stk_scratch(c, 3, tiles * sizeof(unsigned int), &cnt));
-        STK_CUDA(c, cudaMemsetAsync(cnt, 0, tiles * sizeof(unsigned int), s));
-        P.hash_on = 1; P.grid_swap = 1; P.hash_nodes = hash_nodes; P.hash_cnt = (unsigned int*)cnt;
-      }
     }
     if (c->is_stark) STK_TRY(launch_pass<StarkField>(c, s, P, StarkField()));
     else STK_TRY(launch_pass<MontField>(c, s, P, c->mont));
   }
   return STK_OK;
-}
-
-// The final pass can also hash the Merkle bottom level when it is a multi-pass transform over
-// the STARK prime whose tiles fit grid.y and hold whole permute4 quads (k >= 2).
-bool stk_ntt_can_fuse_hash(stk_ctx* c, uint64_t n, uint64_t batch) {
-  if (!c->is_stark || n < 8 || (n & (n - 1)) || batch == 0 || batch > 0x7fffffffull) return false;
-  // Opt-in: measured SLOWER than the separate leaf kernel on B200 (64 x 2^21: 24.4 vs 23.3 ms,
-  // DESIGN.md section 4) -- the pass kernel fills the register file at 16 warps/SM, so hashing
-  // CTAs displace butterfly CTAs instead of filling their idle ALU slots.
-  if (!env_int("STK_FUSED_HASH", 0)) return false;
-  std::vector<NttPass> plan;
-  if (build_plan(ilog2_u64(n), batch, plan, ntt_max_radix()) != STK_OK || plan.size() < 2) return false;
-  const NttPass& L = plan.back();
-  return L.k >= 2 && L.nrounds >= 2 && (n >> L.logT) <= 65535;
-}
-
-int stk_ntt_dev_hash(stk_ctx* c, const fe* d_in, uint64_t n_in, uint64_t in_stride, fe* d_out, uint64_t out_stride,
-                     uint64_t n, uint64_t batch, const fe& root, uint32_t* d_nodes) {
-  return ntt_dev_on(c, c->stream, 0, d_in, n_in, in_stride, d_out, out_stride, n, batch, root, 0, 0, nullptr, d_nodes);
 }
 
 int stk_ntt_dev_peer(stk_ctx* c, const fe* d_in, uint64_t n_in, uint64_t in_stride, uint64_t n, uint64_t batch,
@@ -590,8 +559,8 @@ int stk_ntt_dev_peer(stk_ctx* c, const fe* d_in, uint64_t n_in, uint64_t in_stri
 // (r0: the trace an 8x low-degree extension started from): see NttPass::cskip0.
 int stk_ntt_dev_r0(stk_ctx* c, const fe* d_in, uint64_t n_in, uint64_t in_stride, fe* d_out, uint64_t out_stride,
                    uint64_t n, uint64_t batch, const fe& root, const fe* r0, uint64_t r0_stride) {
-  return ntt_dev_on(c, c->stream, 0, d_in, n_in, in_stride, d_out, out_stride, n, batch, root, 0, 0, nullptr, nullptr,
-                    r0, r0_stride);
+  return ntt_dev_on(c, c->stream, 0, d_in, n_in, in_stride, d_out, out_stride, n, batch, root, 0, 0, nullptr, r0,
+                    r0_stride);
 }
 
 int stk_ntt_dev(stk_ctx* c, const fe* d_in, uint64_t n_in, uint64_t in_stride, fe* d_out, uint64_t out_stride,
@@ -648,8 +617,7 @@ extern "C" __attribute__((visibility("default"))) int stk_ntt_host(stk_ctx* c, c
   fe r = stk_load_fe(root);
   constexpr int kSlots = 3;
   const uint64_t col_bytes = n * sizeof(fe);
-  const uint64_t chunk_target = (uint64_t)std::max(1, env_int("STK_HOST_CHUNK_MB", 64)) << 20;
-  uint64_t chunk = std::max<uint64_t>(1, chunk_target / col_bytes);
+  uint64_t chunk = std::max<uint64_t>(1, ((uint64_t)64 << 20) / col_bytes);  // 64 MiB of output per slot
   chunk = std::min(chunk, batch);
   // slot buffers: in (n_in per column, packed) and out (n per column)
   void* bufs;
@@ -726,7 +694,7 @@ static int dist_phase_impl(stk_ctx* c, int phase, const uint32_t* d_in, uint32_t
   STK_TRY(stk_get_table(c, w, N, &W));
   std::vector<NttPass> plan;
   if (phase == 0) {
-    STK_TRY(build_plan(nloc, batch, plan, c->is_stark ? ntt_max_radix() : 2));
+    STK_TRY(build_plan(nloc, batch, plan, c->is_stark ? kStarkRadix : 2));
     for (auto& P : plan) {
       P.final_pass = 0;  // keep the tile geometry, store in place
       P.n_tw = n; P.j_shift = g; P.j_or = (uint32_t)rank; P.out_shift = 0;
@@ -739,7 +707,7 @@ static int dist_phase_impl(stk_ctx* c, int phase, const uint32_t* d_in, uint32_t
     }
   } else {
     // last g levels: bits [0, g) of the local index; final-pass geometry (batch bits on top)
-    const int logT = std::min(10, std::max(6, env_int("STK_NTT_LOGT", 10)));
+    const int logT = 10;
     NttPass P;
     memset(&P, 0, sizeof P);
     P.n = nloc; P.k = g; P.lo = 0; P.final_pass = 1; P.c_is_col = 0;
@@ -747,7 +715,7 @@ static int dist_phase_impl(stk_ctx* c, int phase, const uint32_t* d_in, uint32_t
     P.cb = nloc - P.logC;
     P.nl = nloc - P.logC - g; P.sl = g; P.sh = 0;
     P.logT = P.k + P.logC;
-    fill_rounds(P, c->is_stark ? ntt_max_radix() : 2);
+    fill_rounds(P, c->is_stark ? kStarkRadix : 2);
     P.n_tw = n; P.j_shift = 0; P.j_or = (uint32_t)(rank << nloc); P.out_shift = g;
     P.in_rot = rotated_input ? g : 0;
     plan.push_back(P);

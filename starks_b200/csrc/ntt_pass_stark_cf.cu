@@ -1,32 +1,9 @@
-// ntt_pass_stark_cf.cu -- final pass of a coset transform (interleaved store), 1024-element tiles; one instantiation per
-// translation unit so the heavy kernels compile in parallel (see ntt_pass_stark.cu).
-#include <algorithm>
-#include "ctx.h"
+// ntt_pass_stark_cf.cu -- one instantiation of the NTT pass kernel (ntt.cuh): final pass of a
+// coset transform (interleaved store), 1024-element tiles.
+// Each instantiation has its own translation unit so that the heavy kernels compile in parallel.
 #include "ntt.cuh"
 
 using namespace stk;
-
-template <class F, int MAXR, int MAXT, int MINB, int ZS>
-static int launch_pass_r(stk_ctx* c, cudaStream_t s, const NttPass& P, const F& f) {
-  static bool attr_done[64] = {};  // cudaFuncSetAttribute is per device
-  if (!attr_done[c->device & 63]) {
-    STK_CUDA(c, cudaFuncSetAttribute(ntt_pass_kernel<F, MAXR, MAXT, MINB, ZS>,
-                                     cudaFuncAttributeMaxDynamicSharedMemorySize, 32 * 8 * MAXT));
-    attr_done[c->device & 63] = true;
-  }
-  const uint32_t T = 1u << P.logT;
-  if ((1u << P.logT) > 8u * MAXT) return stk_fail(c, STK_EUNSUPPORTED, "tile larger than this instantiation");
-  unsigned threads = std::max(1u, T >> MAXR);
-  uint64_t tiles = P.c_is_col ? 1 : ((1ull << P.n) >> P.logT);
-  uint64_t cols = P.c_is_col ? ((P.batch + (1u << P.logC) - 1) >> P.logC) : P.batch;
-  if (!P.c_is_col && cols > 65535) return stk_fail(c, STK_EUNSUPPORTED, "more than 65535 columns of a multi-pass transform");
-  if (cols > 0x7fffffffull) return stk_fail(c, STK_EUNSUPPORTED, "batch too large");
-  dim3 grid(P.c_is_col ? (unsigned)cols : (unsigned)tiles, P.c_is_col ? 1u : (unsigned)cols);
-  size_t smem = (P.nrounds > 1 || P.peer_on) ? (size_t)32 * T : 0;
-  ntt_pass_kernel<F, MAXR, MAXT, MINB, ZS><<<grid, threads, smem, s>>>(P, f);
-  STK_CUDA(c, cudaGetLastError());
-  return STK_OK;
-}
 
 int stk_launch_pass_stark_cf(stk_ctx* c, cudaStream_t s, const NttPass& P) {
   return launch_pass_r<StarkField, 3, 128, 4, 2>(c, s, P, StarkField());

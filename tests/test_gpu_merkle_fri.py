@@ -179,37 +179,6 @@ def test_full_size_commit_properties(eng, oracle):
   assert eng.merkle_commit(d.ptr, n, ncols, n, nodes.ptr) != root
 
 
-def test_fused_leaf_hash_matches_separate_commit(eng, oracle, monkeypatch):
-  """stk_lde_commit hashes the Merkle bottom level inside the transform's final pass when the
-  shape allows it (ntt.cuh, HASH); every node must equal the separate-kernel commit's and the
-  oracle's tree (merkelize_polynomial_evaluations, merkle_tree.py:94-119)."""
-  from starks_b200.limbs import limbs_to_be_bytes
-  rng = np.random.default_rng(23)
-  for steps, ncols in ((1 << 9, 1), (1 << 9, 5), (1 << 12, 3), (1 << 14, 64), (1 << 18, 2), (1 << 19, 1)):
-    ext = 8
-    N = steps * ext
-    G2 = pow(7, (P - 1) // N, P)
-    trace = rand_cols(rng, ncols, steps)
-    d_tr = eng.alloc(trace.nbytes).upload(trace)
-    d_ev = eng.alloc(ncols * N * 32)
-    got = {}
-    for fused in ("1", "0"):
-      monkeypatch.setenv("STK_FUSED_HASH", fused)
-      nodes = eng.alloc(32 * N)
-      eng._check(eng.lib.stk_memset(eng.ctx, nodes.ptr, 0xA5, 32 * N))
-      root = eng.lde_commit(d_tr.ptr, steps, steps, ext, ncols, G2, d_ev.ptr, N, nodes.ptr)
-      got[fused] = (root, nodes.download((N, 32), dtype=np.uint8)[1:].copy(), d_ev.download((ncols, N, 8)))
-      nodes.free()
-    assert got["1"][0] == got["0"][0]
-    assert (got["1"][2] == got["0"][2]).all()
-    assert (got["1"][1] == got["0"][1]).all(), "steps=%d cols=%d" % (steps, ncols)
-    if N <= 1 << 15:
-      leaves = np.concatenate([limbs_to_be_bytes(c) for c in got["1"][2]], axis=1)
-      _, want_nodes = oracle.merkelize_bytes(leaves, 4)
-      assert got["1"][0] == want_nodes[1].tobytes()
-    d_tr.free(); d_ev.free()
-
-
 def test_fri_driver_matches_layer_loop(eng, oracle):
   """stk_fri_prove (whole commit phase in the library) must produce the same proof object as the
   per-layer Python loop over the same kernels (starks/fri.py:189-266)."""
