@@ -112,7 +112,10 @@ int stk_ntt_dist_phase0_p2p(stk_ctx* ctx, uint32_t* d_inout, uint64_t local_n, c
 /* ---- LDE ------------------------------------------------------------------------ */
 /* construct_trace_polynomials + evaluation loop (starks/stark.py:27-36, 254-256): per column
  * inverse NTT of `steps` trace values over <G1>, G1 = g2^ext, then forward NTT of the
- * coefficients over <g2> (order steps*ext).  d_coeffs may be NULL (scratch is used). */
+ * coefficients over <g2> (order steps*ext).  d_coeffs may be NULL (scratch is used), or equal
+ * to d_trace with coeff_stride == trace_stride: the coefficients then replace the trace (with
+ * ext = 8 the evaluations are computed in full instead of copying residue 0 from the trace).
+ * Any other overlap of the coefficient rows with the trace rows returns STK_EINVAL. */
 int stk_lde(stk_ctx* ctx, const uint32_t* d_trace, uint64_t steps, uint64_t trace_stride, uint64_t ext,
             uint64_t cols, const uint32_t g2[8], uint32_t* d_coeffs, uint64_t coeff_stride, uint32_t* d_evals,
             uint64_t eval_stride);

@@ -21,6 +21,14 @@ STK_API int stk_lde(stk_ctx* c, const uint32_t* d_trace, uint64_t steps, uint64_
                     uint64_t eval_stride) {
   if (!c || !d_trace || !d_evals || !g2 || steps == 0 || ext == 0 || cols == 0) return STK_EINVAL;
   const uint64_t n = steps * ext;
+  // The coefficients may replace the trace in its own buffer (same start and stride: the inverse
+  // transform runs in place); any other overlap would overwrite trace values still to be read.
+  const bool in_place = (const void*)d_coeffs == (const void*)d_trace && coeff_stride == trace_stride;
+  if (d_coeffs && !in_place) {
+    const uint64_t t0 = (uint64_t)d_trace, t1 = t0 + ((cols - 1) * trace_stride + steps) * sizeof(fe);
+    const uint64_t c0 = (uint64_t)d_coeffs, c1 = c0 + ((cols - 1) * coeff_stride + steps) * sizeof(fe);
+    if (c0 < t1 && t0 < c1) return stk_fail(c, STK_EINVAL, "coefficient rows overlap the trace rows");
+  }
   fe G2 = stk_load_fe(g2);
   fe G1 = stk_h_pow(c, G2, ext);
   fe* coef = (fe*)d_coeffs;
@@ -32,8 +40,9 @@ STK_API int stk_lde(stk_ctx* c, const uint32_t* d_trace, uint64_t steps, uint64_
   }
   STK_TRY(stk_ntt_dev(c, (const fe*)d_trace, steps, trace_stride, coef, coeff_stride, steps, cols, G1, 1, 1));
   // ext = 8: evals[8K] = trace[K] (the evaluation domain contains the trace domain unshifted), so
-  // the residue-0 coset of the forward transform is copied instead of computed
-  if (ext == 8 && c->is_stark && (const void*)d_trace != (const void*)d_evals)
+  // the residue-0 coset of the forward transform is copied instead of computed -- unless the
+  // coefficients have just overwritten the trace
+  if (ext == 8 && c->is_stark && !in_place && (const void*)d_trace != (const void*)d_evals)
     return stk_ntt_dev_r0(c, coef, steps, coeff_stride, (fe*)d_evals, eval_stride, n, cols, G2, (const fe*)d_trace,
                           trace_stride);
   STK_TRY(stk_ntt_dev(c, coef, steps, coeff_stride, (fe*)d_evals, eval_stride, n, cols, G2, 0, 0));
