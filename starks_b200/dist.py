@@ -482,8 +482,7 @@ class ShardedProver(object):
     on rank 0 (None elsewhere)."""
     import time
     from .fri import FRI, DeviceLayer
-    from .limbs import limbs_to_ints
-    from .stark import get_pseudorandom_ks
+    from .stark import interleave_branches, lincomb_weights
     from .utils import get_pseudorandom_indices
     t0 = time.perf_counter()
     marks = []
@@ -495,16 +494,10 @@ class ShardedProver(object):
     G2 = int(S.G2)
     if isinstance(self.comm, NcclComm):
       _adopt_stream(eng, self.rows)   # order the engine's kernels with torch's collectives
-    tr = S._witness_limbs(witness)
-    on_device = not isinstance(tr, np.ndarray)      # a DevBuf (air.witness_device): nothing to upload
-    if on_device:
-      d_trace = tr
-      last_rows = np.stack([d_trace.download((1, 8), byte_offset=(j * steps + steps - 1) * 32)[0] for j in range(w)])
-    else:
-      d_trace = eng.alloc(w * steps * 32).upload(tr, wait=False)
-      last_rows = tr[:, -1, :]
+    d_trace, owned, noncanonical = S._witness(eng, witness)
     c0, c1 = split_columns(3 * w, G)[rank]
-    d_coef, cs = S.coefficient_rows(eng, d_trace.ptr, boundary, limbs_to_ints(last_rows), want=range(c0, c1))
+    d_coef, cs = S.coefficient_rows(eng, d_trace.ptr, boundary, S._last_row(witness), want=range(c0, c1),
+                                    witness_check=noncanonical)
     mark("coefficients")
     self.comm.rows_barrier(eng, 0)       # nobody still reads the previous proof's rows
     eng.ntt_p2p(d_coef.at(c0 * cs * 32), cs, cs, N, c1 - c0, G2, G, c0, self.ptrs)
@@ -512,16 +505,8 @@ class ShardedProver(object):
     top_m = combine_subtree_roots(self.comm.commit_roots(eng, self.rows, self.n_local, 3 * w, self.nodes_m))
     m_root = top_m[1]
     mark("m_root")
-    k1, k2, k3, k4 = get_pseudorandom_ks(m_root, 4)
-    l_ks = get_pseudorandom_ks(m_root, w)
-    c = pow(pow(G2, steps, p), N - 1, p)
-    wP, wD, wB = [], [], []
-    for j in range(w):
-      aj = (1 + l_ks[j] * c) % p
-      wD.append(aj)
-      wP.append(aj * ((k1 + k2 * c) % p) % p)
-      wB.append(aj * ((k3 + k4 * c) % p) % p)
-    eng.lincomb(self.rows.data_ptr(), self.n_local, 3 * w, self.n_local, wP + wD + wB, self.l_rows.data_ptr())
+    eng.lincomb(self.rows.data_ptr(), self.n_local, 3 * w, self.n_local, lincomb_weights(m_root, w, steps, N, G2, p),
+                self.l_rows.data_ptr())
     top_l = combine_subtree_roots(self.comm.commit_roots(eng, self.l_rows, self.n_local, 1, self.nodes_l))
     l_root = top_l[1]
     mark("l_root")
@@ -541,9 +526,7 @@ class ShardedProver(object):
         (self.rows, 3 * w, self.nodes_m, top_m, [x for pos in positions for x in (pos, (pos + ext) % N)]),
         (self.l_rows, 1, self.nodes_l, top_l, positions),
         (self.l_rows, 1, self.nodes_l, top_l, [y + q * j for y in ys for j in range(4)])])
-    branches = []
-    for i in range(len(positions)):
-      branches += [mb[2 * i], mb[2 * i + 1], lb[i]]
+    branches = interleave_branches(mb, lb)
     mark("fri_layer0_and_branches")
     proof = None
     if rank == 0:
@@ -555,7 +538,7 @@ class ShardedProver(object):
       proof = [m_root, l_root, branches, fri_proof]
     mark("fri_rest")
     eng.sync()
-    if not on_device:
+    if owned:
       d_trace.free()
     d_coef.free()
     self.timings = {"mk_proof_s": time.perf_counter() - t0}

@@ -115,6 +115,9 @@ class Engine:
   def close(self):
     if self.ctx is not None:
       self.release_pool()
+      if self._flag is not None:
+        self._flag.free()
+        self._flag = None
       self.lib.stk_destroy(self.ctx)
       self.ctx = None
 

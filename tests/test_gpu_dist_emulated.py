@@ -208,3 +208,45 @@ def test_sharded_prover_emulated(oracle, world, logsteps, air):
   assert not errors, errors
   assert results[0] == want, "sharded proof differs from the one-GPU proof"
   assert all(x is None for x in results[1:])
+
+
+@pytest.mark.parametrize("world", [2, 8])
+def test_sharded_prover_rejects_noncanonical_limbs_emulated(oracle, world):
+  """Limbs >= p are not field elements: every rank of the sharded prover refuses them with the
+  error STARK.mk_proof raises, whether it derives D rows (whose divisibility check would fail
+  first), only P or B rows, or none (8 ranks, 6 rows)."""
+  import threading
+  import torch
+  from starks_b200 import Engine
+  from starks_b200.dist import ShardedProver, ThreadComm
+  from starks_b200.limbs import ints_to_limbs
+  from starks_b200.modp import IntegersModP
+  steps, width, sp, inp = 1 << 9, 2, [{(0, 1): 1}, {(1, 0): 1, (0, 1): 1}], [0, 1]
+  bad = np.stack([ints_to_limbs(col) for col in oracle.computational_trace(P, inp, steps, sp)])
+  bad[1, 5] = np.array([0xFFFFFFFF] * 8, dtype=np.uint32)
+  bnd = [(0, j, inp[j]) for j in range(width)]
+  dev = torch.device("cuda", 0)
+  shared = ThreadComm.Shared(world)
+  outcome = [None] * world
+
+  def run(r):
+    try:
+      torch.cuda.set_device(0)
+      eng = Engine(0)
+      prover = ShardedProver(eng, IntegersModP(P), steps, 8, width, sp, dev, comm=ThreadComm(shared, r, dev))
+      try:
+        prover.mk_proof(bad, bnd)
+        outcome[r] = "returned"
+      except ValueError as ex:
+        outcome[r] = str(ex)
+      eng.close()
+    except BaseException as ex:  # noqa: BLE001
+      outcome[r] = repr(ex)
+      shared.bar.abort()
+
+  threads = [threading.Thread(target=run, args=(r,)) for r in range(world)]
+  for t in threads:
+    t.start()
+  for t in threads:
+    t.join(timeout=600)
+  assert outcome == ["witness holds elements >= p; reduce them mod p first"] * world, outcome
