@@ -86,6 +86,22 @@ int stk_ntt_host(stk_ctx* ctx, const uint32_t* h_in, uint64_t n_in, uint64_t in_
  * WITHOUT the 1/n scaling, exactly as the reference. */
 int stk_mul_polys(stk_ctx* ctx, const uint32_t* d_a, uint64_t na, const uint32_t* d_b, uint64_t nb,
                   uint32_t* d_out, uint64_t n, const uint32_t root[8]);
+/* Polynomial.__mul__ (starks/polynomial.py:110-121): d_out[0 .. na+nb-1) = a * b (linear, not
+ * cyclic; coefficients low -> high).  na == 0 or nb == 0 writes nothing.  d_out must not
+ * overlap either input (STK_EINVAL).  Asynchronous.  Forward transforms, a pointwise product and
+ * a scaled inverse where Z/p has a root of unity of the power-of-two order the product needs
+ * (the STARK prime always; otherwise z^((p-1)/L) for a quadratic non-residue z); a direct
+ * O(na*nb) kernel where it has none (e.g. p = 31).  Products longer than 2^30: STK_EUNSUPPORTED. */
+int stk_poly_mul(stk_ctx* ctx, const uint32_t* d_a, uint64_t na, const uint32_t* d_b, uint64_t nb,
+                 uint32_t* d_out);
+/* Polynomial.__divmod__ (starks/polynomial.py:128-143): a = b*q + r with deg r < deg b.
+ * d_q receives max(na-nb+1, 0) coefficients; d_r receives nb-1 (zero-padded when na < nb-1).
+ * nb >= 1 and b[nb-1] != 0, otherwise STK_EINVAL.  The call reads b's leading coefficient,
+ * so it synchronises the stream.  Outputs must not overlap inputs or each other.  Newton
+ * iteration on the reversed divisor (g <- g(2 - f g), doubling the precision), with products
+ * routed as in stk_poly_mul. */
+int stk_poly_divmod(stk_ctx* ctx, const uint32_t* d_a, uint64_t na, const uint32_t* d_b, uint64_t nb,
+                    uint32_t* d_q, uint32_t* d_r);
 /* Pointwise helpers on device columns: out[i] = a[i] (op) b[i]; op 0 add, 1 sub, 2 mul. */
 int stk_vec_op(stk_ctx* ctx, int op, const uint32_t* d_a, const uint32_t* d_b, uint32_t* d_out, uint64_t n);
 /* get_power_cycle (starks/utils.py:30-38): out[i] = r^i, i < n (n = order of r). */

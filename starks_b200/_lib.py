@@ -46,6 +46,8 @@ SIGNATURES = {
     "stk_dft_generic": (cint, [vp, vp, u64, u64, vp, u64, u64, u64, u32p, cint]),
     "stk_ntt_host": (cint, [vp, vp, u64, u64, vp, u64, u64, u64, u32p, cint]),
     "stk_mul_polys": (cint, [vp, vp, u64, vp, u64, vp, u64, u32p]),
+    "stk_poly_mul": (cint, [vp, vp, u64, vp, u64, vp]),
+    "stk_poly_divmod": (cint, [vp, vp, u64, vp, u64, vp, vp]),
     "stk_vec_op": (cint, [vp, cint, vp, vp, vp, u64]),
     "stk_power_cycle": (cint, [vp, u32p, u64, vp]),
     "stk_ntt_dist_phase": (cint, [vp, cint, vp, vp, u64, u64, u64, u32p, u64, u64, cint]),

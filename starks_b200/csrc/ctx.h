@@ -55,9 +55,10 @@ struct stk_ctx {
   std::vector<stk_invtable> invtables; // least recently used first
   std::vector<stk_ntt_consts> ntt_consts;
   uint64_t table_gen = 0;  // bumped whenever a table is freed
-  static const int kScratchSlots = 12;
+  static const int kScratchSlots = 14;
   void* scratch[kScratchSlots] = {};   // 0-1 transforms, 2-3 small staging, 4-7 host pipeline, 8-9 FRI,
-  uint64_t scratch_bytes[kScratchSlots] = {};  // 10 device-side counters, 11 host-trace staging
+  uint64_t scratch_bytes[kScratchSlots] = {};  // 10 device-side counters, 11 host-trace staging,
+                                               // 12-13 polynomial product / division (poly.cu)
   std::string err;
 };
 

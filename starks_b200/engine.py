@@ -196,6 +196,16 @@ class Engine:
       x.free()
     return out
 
+  def poly_mul(self, d_a, na, d_b, nb, d_out):
+    """Linear product of two coefficient vectors on the device (stk_poly_mul): d_out receives
+    na + nb - 1 coefficients."""
+    self._check(self.lib.stk_poly_mul(self.ctx, d_a, na, d_b, nb, d_out))
+
+  def poly_divmod(self, d_a, na, d_b, nb, d_q, d_r):
+    """Long division a = b*q + r on the device (stk_poly_divmod): d_q receives max(na-nb+1, 0)
+    coefficients, d_r receives nb-1.  Synchronises the stream."""
+    self._check(self.lib.stk_poly_divmod(self.ctx, d_a, na, d_b, nb, d_q, d_r))
+
   def power_cycle(self, r, n):
     do = self.alloc(n * 32)
     self._check(self.lib.stk_power_cycle(self.ctx, _u32(int_to_limbs(int(r) % self.p)), n, do.ptr))

@@ -1,10 +1,21 @@
 """Minimal dense-polynomial value types mirroring what the hot path touches of
 starks/polynomial.py (coefficient list low -> high, trailing zeros stripped, :58; Horner
-__call__, :158-164) and of starks/multivariate_polynomial.py (dict monomial -> coefficient,
-__call__ :329-338).  Host-side glue only."""
+__call__, :158-164; products and long division, :110-143) and of
+starks/multivariate_polynomial.py (dict monomial -> coefficient, __call__ :329-338).  Products
+and divisions run on the device (stk_poly_mul, stk_poly_divmod); the rest is host-side glue."""
 import functools
+import itertools
 
+from .engine import default_engine
+from .limbs import ints_to_limbs, limbs_to_ints
 from .modp import element_to_int
+
+
+def _upload(eng, coeffs):
+  buf = eng.alloc(max(len(coeffs), 1) * 32)
+  if coeffs:
+    buf.upload(ints_to_limbs(element_to_int(x) for x in coeffs))
+  return buf
 
 
 @functools.lru_cache(maxsize=None)
@@ -48,6 +59,69 @@ def polynomials_over(ring):
       for c in reversed(self.coefficients):
         acc = acc * x + c
       return acc
+
+    @staticmethod
+    def _lift(other):
+      """Anything the constructor accepts: an int or a field element is a constant."""
+      return other if isinstance(other, Polynomial) else Polynomial(other)
+
+    def __add__(self, other):
+      o = Polynomial._lift(other)
+      zero = ring(0)
+      return Polynomial([x + y for x, y in itertools.zip_longest(self.coefficients, o.coefficients,
+                                                                  fillvalue=zero)])
+    __radd__ = __add__
+
+    def __neg__(self):
+      return Polynomial([-x for x in self.coefficients])
+
+    def __sub__(self, other):
+      return self + (-Polynomial._lift(other))
+
+    def __rsub__(self, other):
+      return Polynomial._lift(other) + (-self)
+
+    @staticmethod
+    def _engine():
+      eng = default_engine()
+      eng.set_field(ring.p)
+      return eng
+
+    @staticmethod
+    def _download(buf, n):
+      return Polynomial([ring(v) for v in limbs_to_ints(buf.download((n, 8)))])
+
+    def __mul__(self, other):                        # polynomial.py:110-121, stk_poly_mul
+      o = Polynomial._lift(other)
+      na, nb = len(self), len(o)
+      if not na or not nb:
+        return Polynomial([])
+      eng = Polynomial._engine()
+      da, db = _upload(eng, self.coefficients), _upload(eng, o.coefficients)
+      dout = eng.alloc((na + nb - 1) * 32)
+      try:
+        eng.poly_mul(da.ptr, na, db.ptr, nb, dout.ptr)
+        return Polynomial._download(dout, na + nb - 1)
+      finally:
+        for x in (da, db, dout):
+          x.free()
+    __rmul__ = __mul__
+
+    def __divmod__(self, divisor):                   # polynomial.py:128-143, stk_poly_divmod
+      d = Polynomial._lift(divisor)
+      if d.is_zero():
+        raise ZeroDivisionError("polynomial division by zero")
+      na, nb = len(self), len(d)
+      nq, nr = max(na - nb + 1, 0), nb - 1
+      eng = Polynomial._engine()
+      da, db = _upload(eng, self.coefficients), _upload(eng, d.coefficients)
+      dq, dr = eng.alloc(max(nq, 1) * 32), eng.alloc(max(nr, 1) * 32)
+      try:
+        eng.poly_divmod(da.ptr, na, db.ptr, nb, dq.ptr, dr.ptr)
+        return Polynomial._download(dq, nq), Polynomial._download(dr, nr)
+      finally:
+        for x in (da, db, dq, dr):
+          x.free()
 
     def __repr__(self):
       return "Polynomial(%r)" % ([int(c) for c in self.coefficients],)
