@@ -102,6 +102,33 @@ int stk_poly_mul(stk_ctx* ctx, const uint32_t* d_a, uint64_t na, const uint32_t*
  * routed as in stk_poly_mul. */
 int stk_poly_divmod(stk_ctx* ctx, const uint32_t* d_a, uint64_t na, const uint32_t* d_b, uint64_t nb,
                     uint32_t* d_q, uint32_t* d_r);
+/* Polynomial.__call__ on a polynomial (starks/polynomial.py:158-164): d_out[0 .. (na-1)(nb-1)+1)
+ * = a(b(X)).  na == 0 writes nothing; nb < 2 returns STK_EINVAL (a constant b is a scalar
+ * evaluation).  d_out must not overlap either input (STK_EINVAL); an output longer than 2^30
+ * returns STK_EUNSUPPORTED and writes nothing.  With nb == 2 the call reads b[0] and b[1], so it
+ * synchronises the stream; b = alpha X (b[0] == 0, the prover's P(G1 X)) is then one pointwise
+ * kernel, out[k] = a[k] alpha^k.  Any other b: divide and conquer over a padded to a power of two,
+ * r_i <- r_2i + b^(2^j) r_2i+1 per level, each level one batched forward transform, a broadcast
+ * pointwise product, one batched inverse and an add; levels without a root of the needed order
+ * run through the products of stk_poly_mul (direct kernel).  Asynchronous for nb > 2. */
+int stk_poly_compose(stk_ctx* ctx, const uint32_t* d_a, uint64_t na, const uint32_t* d_b, uint64_t nb,
+                     uint32_t* d_out);
+/* MultivariatePolynomial.__call__ on polynomials (starks/multivariate_polynomial.py:329-338):
+ * argument k has h_lens[k] coefficients at d_polys + 8*k*in_stride (k < width <= 12, else
+ * STK_EUNSUPPORTED).  Monomial m contributes coeffs[m] * prod_k X_k^exps[m*width+k] to output
+ * h_mono_out[m] < nout (the list form of stk_constraint_eval with uint32 exponents).  An exponent
+ * of 0 is a factor of 1 even on an empty argument; a positive one on an empty argument makes the
+ * monomial vanish.  D = max over the remaining monomials of sum_k e_k (h_lens[k] - 1) (0 if none);
+ * out_len must equal D + 1 (STK_EINVAL otherwise), D + 1 > 2^30 returns STK_EUNSUPPORTED.
+ * Output j is written at d_out + 8*j*out_len, zero-padded; outputs must not overlap an argument.
+ * Transform route (a root of order L = 2^ceil(log2(D+1)) exists): one batched forward transform of
+ * the arguments, one pointwise kernel (every monomial by square-and-multiply), one batched scaled
+ * inverse.  Otherwise the monomials are built from stk_poly_mul products.  Synchronises the stream
+ * once to stage the monomial list. */
+int stk_poly_eval_multivar(stk_ctx* ctx, const uint32_t* d_polys, const uint64_t* h_lens, uint64_t in_stride,
+                           uint64_t width, const uint32_t* h_mono_out, const uint32_t* h_mono_coeffs,
+                           const uint32_t* h_mono_exps, uint64_t nmono, uint64_t nout, uint32_t* d_out,
+                           uint64_t out_len);
 /* Pointwise helpers on device columns: out[i] = a[i] (op) b[i]; op 0 add, 1 sub, 2 mul. */
 int stk_vec_op(stk_ctx* ctx, int op, const uint32_t* d_a, const uint32_t* d_b, uint32_t* d_out, uint64_t n);
 /* get_power_cycle (starks/utils.py:30-38): out[i] = r^i, i < n (n = order of r). */

@@ -48,6 +48,8 @@ SIGNATURES = {
     "stk_mul_polys": (cint, [vp, vp, u64, vp, u64, vp, u64, u32p]),
     "stk_poly_mul": (cint, [vp, vp, u64, vp, u64, vp]),
     "stk_poly_divmod": (cint, [vp, vp, u64, vp, u64, vp, vp]),
+    "stk_poly_compose": (cint, [vp, vp, u64, vp, u64, vp]),
+    "stk_poly_eval_multivar": (cint, [vp, vp, vp, u64, u64, vp, vp, vp, u64, u64, vp, u64]),
     "stk_vec_op": (cint, [vp, cint, vp, vp, vp, u64]),
     "stk_power_cycle": (cint, [vp, u32p, u64, vp]),
     "stk_ntt_dist_phase": (cint, [vp, cint, vp, vp, u64, u64, u64, u32p, u64, u64, cint]),

@@ -11,7 +11,7 @@ import threading
 import numpy as np
 
 from . import _lib
-from .limbs import int_to_limbs
+from .limbs import int_to_limbs, ints_to_limbs
 
 P_STARK = 2**256 - 351 * 2**32 + 1
 
@@ -205,6 +205,26 @@ class Engine:
     """Long division a = b*q + r on the device (stk_poly_divmod): d_q receives max(na-nb+1, 0)
     coefficients, d_r receives nb-1.  Synchronises the stream."""
     self._check(self.lib.stk_poly_divmod(self.ctx, d_a, na, d_b, nb, d_q, d_r))
+
+  def poly_compose(self, d_a, na, d_b, nb, d_out):
+    """Composition a(b(X)) on the device (stk_poly_compose): d_out receives (na-1)(nb-1)+1
+    coefficients; nb >= 2.  Synchronises the stream when nb == 2."""
+    self._check(self.lib.stk_poly_compose(self.ctx, d_a, na, d_b, nb, d_out))
+
+  def poly_eval_multivar(self, d_polys, lens, in_stride, monomials, nout, d_out, out_len):
+    """Multivariate polynomials evaluated at polynomials on the device (stk_poly_eval_multivar).
+    Argument k has lens[k] coefficients at d_polys + 32*k*in_stride; monomials is a list of
+    (output index, int coefficient, exponent tuple of len(lens)); output j is written at
+    d_out + 32*j*out_len, and out_len must be D + 1 (see the header)."""
+    width, nmono = len(lens), len(monomials)
+    h_lens = np.asarray(lens, dtype=np.uint64)
+    h_out = np.asarray([m[0] for m in monomials] or [0], dtype=np.uint32)
+    h_coeffs = ints_to_limbs([int(m[1]) % self.p for m in monomials] or [0])
+    h_exps = np.asarray([e for m in monomials for e in m[2]] or [0], dtype=np.uint32)
+    assert h_exps.size == max(nmono * width, 1), "every exponent tuple needs one entry per argument"
+    self._check(self.lib.stk_poly_eval_multivar(self.ctx, d_polys, h_lens.ctypes.data, in_stride, width,
+                                                h_out.ctypes.data, h_coeffs.ctypes.data, h_exps.ctypes.data, nmono,
+                                                nout, d_out, out_len))
 
   def power_cycle(self, r, n):
     do = self.alloc(n * 32)

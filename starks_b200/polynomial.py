@@ -1,10 +1,14 @@
 """Minimal dense-polynomial value types mirroring what the hot path touches of
 starks/polynomial.py (coefficient list low -> high, trailing zeros stripped, :58; Horner
 __call__, :158-164; products and long division, :110-143) and of
-starks/multivariate_polynomial.py (dict monomial -> coefficient, __call__ :329-338).  Products
-and divisions run on the device (stk_poly_mul, stk_poly_divmod); the rest is host-side glue."""
+starks/multivariate_polynomial.py (dict monomial -> coefficient, __call__ :329-338).  Products,
+divisions, composition, powers and multivariate polynomials evaluated at polynomials run on the
+device (stk_poly_mul, stk_poly_divmod, stk_poly_compose, stk_poly_eval_multivar); the rest is
+host-side glue."""
 import functools
 import itertools
+
+import numpy as np
 
 from .engine import default_engine
 from .limbs import ints_to_limbs, limbs_to_ints
@@ -18,9 +22,47 @@ def _upload(eng, coeffs):
   return buf
 
 
+class _Polynomial(object):
+  """Common base of the classes polynomials_over makes, so that MultiVarPoly can tell a
+  polynomial argument from a constant."""
+
+
+def _out_len(lens, monomials):
+  """D + 1 of stk_poly_eval_multivar: D = max over the monomials that do not vanish (no positive
+  exponent on an empty argument) of sum_k e_k (len_k - 1), 0 if none."""
+  D = 0
+  for _, _, exps in monomials:
+    if not any(e and not n for e, n in zip(exps, lens)):
+      D = max(D, sum(e * (n - 1) for e, n in zip(exps, lens) if e))
+  return D + 1
+
+
+def _eval_multivar(poly_cls, args, monomials, nout):
+  """Device evaluation of nout multivariate polynomials (monomials: (output, int coefficient,
+  exponent tuple)) at the polynomial arguments args; returns nout poly_cls."""
+  lens = [len(a) for a in args]
+  stride = max(lens + [1])
+  out_len = _out_len(lens, monomials)
+  eng = poly_cls._engine()
+  buf = eng.alloc(len(args) * stride * 32)
+  dout = eng.alloc(max(nout, 1) * out_len * 32)
+  try:
+    rows = np.zeros((len(args), stride, 8), dtype=np.uint32)
+    for k, a in enumerate(args):
+      if lens[k]:
+        rows[k, :lens[k]] = ints_to_limbs(element_to_int(x) for x in a.coefficients)
+    buf.upload(rows)
+    eng.poly_eval_multivar(buf.ptr, lens, stride, monomials, nout, dout.ptr, out_len)
+    got = limbs_to_ints(dout.download((nout, out_len, 8)).reshape(-1, 8)) if nout else []
+    return [poly_cls([poly_cls.ring(v) for v in got[j * out_len:(j + 1) * out_len]]) for j in range(nout)]
+  finally:
+    buf.free()
+    dout.free()
+
+
 @functools.lru_cache(maxsize=None)
 def polynomials_over(ring):
-  class Polynomial(object):
+  class Polynomial(_Polynomial):
     def __init__(self, c):
       if isinstance(c, Polynomial):
         coeffs = list(c.coefficients)
@@ -55,10 +97,33 @@ def polynomials_over(ring):
       return [int(x) for x in self.coefficients] == [element_to_int(x) for x in oc]
 
     def __call__(self, x):                           # polynomial.py:158-164
+      if isinstance(x, Polynomial):                  # a(x(X)): stk_poly_compose
+        if len(x) < 2:
+          return Polynomial([self(x.coefficients[0] if len(x) else ring(0))])
+        na, nb = len(self), len(x)
+        if not na:
+          return Polynomial([])
+        eng = Polynomial._engine()
+        da, db = _upload(eng, self.coefficients), _upload(eng, x.coefficients)
+        n = (na - 1) * (nb - 1) + 1
+        dout = eng.alloc(n * 32)
+        try:
+          eng.poly_compose(da.ptr, na, db.ptr, nb, dout.ptr)
+          return Polynomial._download(dout, n)
+        finally:
+          for b in (da, db, dout):
+            b.free()
       acc = ring(0)
       for c in reversed(self.coefficients):
         acc = acc * x + c
       return acc
+
+    def __pow__(self, e):                            # one variable, one monomial: stk_poly_eval_multivar
+      if not isinstance(e, int):
+        return NotImplemented
+      if e < 0:
+        raise ValueError("a polynomial has no negative powers")
+      return _eval_multivar(Polynomial, [self], [(0, 1, (e,))], 1)[0]
 
     @staticmethod
     def _lift(other):
@@ -179,6 +244,8 @@ class MultiVarPoly(object):
 
   def __call__(self, vals):                          # multivariate_polynomial.py:329-338
     assert len(vals) == self.num_vars
+    if any(isinstance(v, _Polynomial) for v in vals):
+      return eval_at_polynomials([self], vals)[0]
     y = self.field(0)
     for k in sorted(self.coefficients):
       prod = self.field(1)
@@ -186,6 +253,18 @@ class MultiVarPoly(object):
         prod = prod * vals[i]**power
       y = y + self.coefficients[k] * prod
     return y
+
+
+def eval_at_polynomials(mvps, polys):
+  """[m(polys) for m in mvps] in one device call (stk_poly_eval_multivar): the reference's
+  step_j(P_1, ..., P_w) for every j (starks/stark.py:49).  At least one of polys is a Polynomial;
+  ints and field elements among them are constants.  Returns Polynomials of that class."""
+  poly_cls = next(type(v) for v in polys if isinstance(v, _Polynomial))
+  args = [v if isinstance(v, poly_cls) else poly_cls(v) for v in polys]
+  monomials = []
+  for j, m in enumerate(mvps):
+    monomials += [(j, c, exps) for exps, c in monomials_of(m, len(args), poly_cls.ring.p)]
+  return _eval_multivar(poly_cls, args, monomials, len(mvps))
 
 
 def generate_Xi_s(field, width):
