@@ -50,24 +50,18 @@ static int fri_fold4_launch(stk_ctx* c, const uint32_t* d_vals, uint64_t n, cons
   STK_TRY(stk_get_table_strided(c, winv, n, &Winv, &wstride));
   fe iota_tw = stk_h_to_tw(c, stk_h_pow(c, w, q));
   unsigned blocks = (unsigned)((q_run + 255) / 256);
-  if (c->is_stark)
-    fri_fold4_kernel<StarkField><<<blocks, 256, 0, c->stream>>>((const fe*)d_vals, q_run, i0, Winv, wstride, x, iota_tw,
-                                                                quarter_tw, (fe*)d_out, StarkField());
-  else
-    fri_fold4_kernel<MontField><<<blocks, 256, 0, c->stream>>>((const fe*)d_vals, q_run, i0, Winv, wstride, x, iota_tw,
-                                                               quarter_tw, (fe*)d_out, c->mont);
-  STK_CUDA(c, cudaGetLastError());
-  return STK_OK;
+  return stk_with_field(c, [&](auto f) {
+    fri_fold4_kernel<<<blocks, 256, 0, c->stream>>>((const fe*)d_vals, q_run, i0, Winv, wstride, x, iota_tw, quarter_tw,
+                                                    (fe*)d_out, f);
+  });
 }
 
-extern "C" __attribute__((visibility("default"))) int stk_fri_fold4(stk_ctx* c, const uint32_t* d_vals, uint64_t n,
-                                                                     const uint32_t root[8], const uint32_t special_x[8],
-                                                                     uint32_t* d_out) {
+STK_API int stk_fri_fold4(stk_ctx* c, const uint32_t* d_vals, uint64_t n, const uint32_t root[8],
+                          const uint32_t special_x[8], uint32_t* d_out) {
   if (!c || !d_vals || !d_out || !root || !special_x) return STK_EINVAL;
   if (n == 0 || (n & 3)) return stk_fail(c, STK_EINVAL, "fold-by-4 needs a length divisible by 4");
   fe w = stk_load_fe(root);
-  fe one = host::reduce(host::from_u64(1), c->p);
-  if (!fe_eq(stk_h_pow(c, w, n), one) || fe_eq(stk_h_pow(c, w, n / 2), one))
+  if (!stk_h_primitive(c, w, n))
     return stk_fail(c, STK_EINVAL, "root is not a primitive n-th root of unity");
   fe x = host::reduce(stk_load_fe(special_x), c->p);  // fri.py:229 does not reduce; products do
   fe quarter_tw = stk_h_to_tw(c, stk_h_inv(c, host::reduce(host::from_u64(4), c->p)));
@@ -78,15 +72,13 @@ extern "C" __attribute__((visibility("default"))) int stk_fri_fold4(stk_ctx* c, 
 // aligned to fold quads"): d_rows holds the four runs {j*q + i0 + t : t < q_run}, j < 4, of the
 // n-point layer back to back (the row order of a rank's local tree under permute4), d_out
 // receives column[i0 .. i0 + q_run).
-extern "C" __attribute__((visibility("default"))) int stk_fri_fold4_rows(stk_ctx* c, const uint32_t* d_rows, uint64_t n,
-                                                                          const uint32_t root[8], const uint32_t special_x[8],
-                                                                          uint64_t q_run, uint64_t i0, uint32_t* d_out) {
+STK_API int stk_fri_fold4_rows(stk_ctx* c, const uint32_t* d_rows, uint64_t n, const uint32_t root[8],
+                               const uint32_t special_x[8], uint64_t q_run, uint64_t i0, uint32_t* d_out) {
   if (!c || !d_rows || !d_out || !root || !special_x) return STK_EINVAL;
   if (n == 0 || (n & 3) || q_run == 0 || i0 + q_run > n / 4)
     return stk_fail(c, STK_EINVAL, "fold-by-4 rows: need n divisible by 4 and i0 + q_run <= n/4");
   fe w = stk_load_fe(root);
-  fe one = host::reduce(host::from_u64(1), c->p);
-  if (!fe_eq(stk_h_pow(c, w, n), one) || fe_eq(stk_h_pow(c, w, n / 2), one))
+  if (!stk_h_primitive(c, w, n))
     return stk_fail(c, STK_EINVAL, "root is not a primitive n-th root of unity");
   fe x = host::reduce(stk_load_fe(special_x), c->p);
   fe quarter_tw = stk_h_to_tw(c, stk_h_inv(c, host::reduce(host::from_u64(4), c->p)));
@@ -111,9 +103,6 @@ extern "C" __attribute__((visibility("default"))) int stk_fri_fold4_rows(stk_ctx
 #include <vector>
 #include "hostblake2s.h"
 
-extern "C" int stk_merkle_commit(stk_ctx* c, const uint32_t* d_cols, uint64_t n, uint64_t ncols, uint64_t col_stride,
-                                 uint8_t* d_nodes, uint8_t* h_root);
-
 namespace {
 
 // get_pseudorandom_indices (starks/utils.py:60-90)
@@ -137,20 +126,14 @@ int fri_indices(stk_ctx* c, const uint8_t root[32], uint64_t modulus, uint64_t c
   return STK_OK;
 }
 
-uint64_t rec_bytes_for(uint64_t n) {
-  uint32_t depth = 0;
-  while ((1ull << depth) < n) ++depth;
-  return 64 + 32ull * (depth - 1);
-}
+uint64_t rec_bytes_for(uint64_t n) { return 64 + 32ull * (stk_ilog2(n) - 1); }
 
 }  // namespace
 
 // get_pseudorandom_indices (starks/utils.py:60-90) exactly as the FRI driver derives them; needs no
 // device (ctx may be NULL), so the host BLAKE2s and the index rule are testable on a CPU-only box.
-extern "C" __attribute__((visibility("default"))) int stk_pseudorandom_indices(stk_ctx* c, const uint8_t entropy[32],
-                                                                                uint64_t modulus, uint64_t count,
-                                                                                uint64_t exclude_multiples_of,
-                                                                                uint64_t* h_out) {
+STK_API int stk_pseudorandom_indices(stk_ctx* c, const uint8_t entropy[32], uint64_t modulus, uint64_t count,
+                                     uint64_t exclude_multiples_of, uint64_t* h_out) {
   if (!entropy || !h_out) return STK_EINVAL;
   if (exclude_multiples_of == 1) return stk_fail(c, STK_EINVAL, "exclude_multiples_of = 1 leaves no positions");
   std::vector<uint64_t> v;
@@ -159,10 +142,9 @@ extern "C" __attribute__((visibility("default"))) int stk_pseudorandom_indices(s
   return STK_OK;
 }
 
-extern "C" __attribute__((visibility("default"))) int stk_fri_prove(
-    stk_ctx* c, const uint32_t* d_vals0, uint64_t n0, const uint8_t* d_nodes0, const uint8_t* h_root0,
-    const uint32_t root[8], uint64_t maxdeg_plus_1, uint64_t exclude, uint64_t security, uint8_t* h_out,
-    uint64_t out_cap, uint64_t* out_len) {
+STK_API int stk_fri_prove(stk_ctx* c, const uint32_t* d_vals0, uint64_t n0, const uint8_t* d_nodes0,
+                          const uint8_t* h_root0, const uint32_t root[8], uint64_t maxdeg_plus_1, uint64_t exclude,
+                          uint64_t security, uint8_t* h_out, uint64_t out_cap, uint64_t* out_len) {
   if (!c || !d_vals0 || !root || !h_out || !out_len || (d_nodes0 && !h_root0)) return STK_EINVAL;
   if (n0 < 4 || (n0 & (n0 - 1))) return stk_fail(c, STK_EUNSUPPORTED, "FRI driver needs a power-of-two domain");
   if (exclude == 1) return stk_fail(c, STK_EINVAL, "exclude_multiples_of = 1 leaves no positions");
@@ -187,8 +169,8 @@ extern "C" __attribute__((visibility("default"))) int stk_fri_prove(
   *out_len = total;
   if (out_cap < total) return stk_fail(c, STK_EINVAL, "output buffer too small: need %llu bytes", (unsigned long long)total);
   void *sv, *st;
-  STK_TRY(stk_scratch(c, 8, std::max<uint64_t>(store + (d_nodes0 ? 0 : 32 * n0), 32), &sv));
-  STK_TRY(stk_scratch(c, 9, std::max<uint64_t>(stage, 32), &st));
+  STK_TRY(stk_scratch(c, kSlotFriLayers, std::max<uint64_t>(store + (d_nodes0 ? 0 : 32 * n0), 32), &sv));
+  STK_TRY(stk_scratch(c, kSlotFriStage, std::max<uint64_t>(stage, 32), &st));
   uint8_t* sbase = (uint8_t*)sv;
   uint8_t* stg = (uint8_t*)st;
   const uint32_t* vals = d_vals0;
@@ -201,11 +183,7 @@ extern "C" __attribute__((visibility("default"))) int stk_fri_prove(
     nodes = nb;
   }
   fe w = host::reduce(stk_load_fe(root), c->p);
-  {
-    fe one = host::reduce(host::from_u64(1), c->p);
-    if (!fe_eq(stk_h_pow(c, w, n0), one) || fe_eq(stk_h_pow(c, w, n0 / 2), one))
-      return stk_fail(c, STK_EINVAL, "root is not a primitive n-th root of unity");
-  }
+  if (!stk_h_primitive(c, w, n0)) return stk_fail(c, STK_EINVAL, "root is not a primitive n-th root of unity");
   fe winv = stk_h_inv(c, w);  // layer l folds with w^(4^l): both follow by two squarings
   const fe quarter_tw = stk_h_to_tw(c, stk_h_inv(c, host::reduce(host::from_u64(4), c->p)));
   std::vector<uint8_t> roots(32 * L.size());

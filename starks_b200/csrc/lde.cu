@@ -10,11 +10,6 @@
 
 using namespace stk;
 
-#define STK_API extern "C" __attribute__((visibility("default")))
-
-extern "C" int stk_merkle_commit(stk_ctx* c, const uint32_t* d_cols, uint64_t n, uint64_t ncols, uint64_t col_stride,
-                                 uint8_t* d_nodes, uint8_t* h_root);
-
 // Coefficients (optional output, cols x steps) and evaluations (cols x steps*ext).
 STK_API int stk_lde(stk_ctx* c, const uint32_t* d_trace, uint64_t steps, uint64_t trace_stride, uint64_t ext,
                     uint64_t cols, const uint32_t g2[8], uint32_t* d_coeffs, uint64_t coeff_stride, uint32_t* d_evals,
@@ -34,7 +29,7 @@ STK_API int stk_lde(stk_ctx* c, const uint32_t* d_trace, uint64_t steps, uint64_
   fe* coef = (fe*)d_coeffs;
   if (!coef) {
     void* t;
-    STK_TRY(stk_scratch(c, 1, cols * steps * sizeof(fe), &t));
+    STK_TRY(stk_scratch(c, kSlotLdeCoeffs, cols * steps * sizeof(fe), &t));
     coef = (fe*)t;
     coeff_stride = steps;
   }
@@ -71,15 +66,10 @@ STK_API int stk_lde_p2p(stk_ctx* c, const uint32_t* d_trace, uint64_t steps, uin
   fe G2 = stk_load_fe(g2);
   fe G1 = stk_h_pow(c, G2, ext);
   void* t;
-  STK_TRY(stk_scratch(c, 1, cols * steps * sizeof(fe), &t));
+  STK_TRY(stk_scratch(c, kSlotLdeCoeffs, cols * steps * sizeof(fe), &t));
   fe* coef = (fe*)t;
   STK_TRY(stk_ntt_dev(c, (const fe*)d_trace, steps, trace_stride, coef, steps, steps, cols, G1, 1, 1));
-  stk_peer_leaf peer;
-  peer.g = 0;
-  while ((1ull << peer.g) < nranks) ++peer.g;
-  peer.col0 = (uint32_t)col_base;
-  peer.ptrs = peer_ptrs;
-  return stk_ntt_dev_peer(c, coef, steps, steps, n, cols, G2, peer);
+  return stk_ntt_dev_peer(c, coef, steps, steps, n, cols, G2, nranks, col_base, peer_ptrs);
 }
 
 // Forward transform of COEFFICIENT rows (n_in coefficients each, implicitly zero-padded to n)
@@ -95,12 +85,8 @@ STK_API int stk_ntt_p2p(stk_ctx* c, const uint32_t* d_coeffs, uint64_t n_in, uin
   if (!d_coeffs) return STK_EINVAL;
   if (nranks < 2 || nranks > 8 || (nranks & (nranks - 1))) return stk_fail(c, STK_EINVAL, "2, 4 or 8 ranks");
   if (n & (n - 1)) return stk_fail(c, STK_EINVAL, "the transform length must be a power of two");
-  stk_peer_leaf peer;
-  peer.g = 0;
-  while ((1ull << peer.g) < nranks) ++peer.g;
-  peer.col0 = (uint32_t)col_base;
-  peer.ptrs = peer_ptrs;
-  return stk_ntt_dev_peer(c, (const fe*)d_coeffs, n_in, in_stride, n, cols, stk_load_fe(root), peer);
+  return stk_ntt_dev_peer(c, (const fe*)d_coeffs, n_in, in_stride, n, cols, stk_load_fe(root), nranks, col_base,
+                          peer_ptrs);
 }
 
 // stk_lde_commit with the trace in HOST memory (pinned: stk_host_alloc) -- the end-to-end form of
@@ -129,7 +115,7 @@ STK_API int stk_lde_commit_host(stk_ctx* c, const uint32_t* h_trace, uint64_t st
   }
   const uint64_t slot_cols = std::min(cap, cols);
   void* st;
-  STK_TRY(stk_scratch(c, 11, 2 * slot_cols * col_bytes, &st));
+  STK_TRY(stk_scratch(c, kSlotLdeHost, 2 * slot_cols * col_bytes, &st));
   fe* slot[2] = {(fe*)st, (fe*)st + slot_cols * steps};
   cudaStream_t cp = c->copy_streams[0];
   // the staging slots may still be read by transforms of an earlier call on the compute stream

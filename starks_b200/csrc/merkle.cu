@@ -225,8 +225,7 @@ int reduce_levels(stk_ctx* c, uint32_t* nodes, uint64_t np) {
   for (; lo >= 65536; lo >>= 1)
     merkle_level_kernel<<<(unsigned)((lo + 255) / 256), 256, 0, c->stream>>>(nodes, lo, lo);
   while (lo >= 1024) {                                // lo < 2^16: 2..7 levels at once, down to a 512-node level
-    int loglo = 0;
-    while ((1ull << loglo) < lo) ++loglo;
+    const int loglo = stk_ilog2(lo);
     const int D = loglo - 8 > 7 ? 7 : loglo - 8;      // levels lo, lo/2, ..., lo >> (D-1)
     const uint32_t roots = (uint32_t)(lo >> (D - 1));
     merkle_mid_kernel<<<roots, 64, 0, c->stream>>>(nodes, roots, D);
@@ -238,8 +237,6 @@ int reduce_levels(stk_ctx* c, uint32_t* nodes, uint64_t np) {
 }
 
 }  // namespace
-
-#define STK_API extern "C" __attribute__((visibility("default")))
 
 int stk_merkle_paths_dev(stk_ctx* c, const fe* d_cols, uint64_t n, uint64_t ncols, uint64_t col_stride,
                          const uint8_t* d_nodes, const uint64_t* d_idx, uint64_t k, uint32_t* d_out, uint64_t rec_bytes) {
@@ -314,14 +311,13 @@ STK_API int stk_merkle_paths(stk_ctx* c, const uint32_t* d_cols, uint64_t n, uin
   if (!k) return STK_OK;
   const uint64_t np = 4 * (n / 4);
   if (np == 0 || (np & (np - 1))) return stk_fail(c, STK_EUNSUPPORTED, "branch extraction needs a power-of-two tree");
-  uint32_t depth = 0;
-  while ((1ull << depth) < np) ++depth;
+  const uint32_t depth = stk_ilog2(np);
   const uint64_t need = 2 * 32 * ncols + 32ull * (depth - 1);
   if (rec_bytes < need || (rec_bytes & 3)) return stk_fail(c, STK_EINVAL, "record size %llu < %llu", (unsigned long long)rec_bytes, (unsigned long long)need);
   for (uint64_t i = 0; i < k; ++i)
     if (h_indices[i] >= np) return stk_fail(c, STK_EINDEX, "branch index out of range");
   void* buf;
-  STK_TRY(stk_scratch(c, 2, k * 8 + k * rec_bytes, &buf));
+  STK_TRY(stk_scratch(c, kSlotStage, k * 8 + k * rec_bytes, &buf));
   uint64_t* d_idx = (uint64_t*)buf;
   uint32_t* d_out = (uint32_t*)((char*)buf + k * 8);
   STK_CUDA(c, cudaMemcpyAsync(d_idx, h_indices, k * 8, cudaMemcpyHostToDevice, c->stream));
@@ -343,14 +339,13 @@ STK_API int stk_verify_branches(stk_ctx* c, const uint8_t root[32], uint64_t n, 
   if (!k) return STK_OK;
   if (n < 4 || (n & (n - 1))) return stk_fail(c, STK_EUNSUPPORTED, "branch verification needs a power-of-two tree");
   if (leaf_len == 0 || (leaf_len & 31)) return stk_fail(c, STK_EINVAL, "leaf length must be a multiple of 32 bytes");
-  uint32_t depth = 0;
-  while ((1ull << depth) < n) ++depth;
+  const uint32_t depth = stk_ilog2(n);
   if (rec_bytes != 2 * leaf_len + 32ull * (depth - 1)) return stk_fail(c, STK_EINVAL, "record size does not match the tree depth");
   for (uint64_t i = 0; i < k; ++i)
     if (h_indices[i] >= n) return stk_fail(c, STK_EINDEX, "branch index out of range");
   const uint64_t rb = k * rec_bytes, ib = k * 8;
   void* buf;
-  STK_TRY(stk_scratch(c, 2, rb + ib + 32 + k + 64, &buf));
+  STK_TRY(stk_scratch(c, kSlotStage, rb + ib + 32 + k + 64, &buf));
   uint8_t* base = (uint8_t*)buf;
   uint32_t* d_rec = (uint32_t*)base;
   uint64_t* d_idx = (uint64_t*)(base + ((rb + 7) & ~7ull));

@@ -123,11 +123,11 @@ __global__ void __launch_bounds__(256) field_kernel(fe* out, const fe* in, uint6
 
 }  // namespace
 
-extern "C" __attribute__((visibility("default"))) int stk_microbench(stk_ctx* c, int which, uint64_t iters, float* ms, double* ops) {
+STK_API int stk_microbench(stk_ctx* c, int which, uint64_t iters, float* ms, double* ops) {
   if (!c || !ms || !ops || which < 0 || which > 13) return STK_EINVAL;
   const unsigned blocks = (unsigned)c->sm_count * 8, threads = 256;
   void* buf;
-  STK_TRY(stk_scratch(c, 2, (uint64_t)blocks * threads * sizeof(fe) + 1024 * sizeof(fe), &buf));
+  STK_TRY(stk_scratch(c, kSlotStage, (uint64_t)blocks * threads * sizeof(fe) + 1024 * sizeof(fe), &buf));
   fe* out = (fe*)buf;
   fe* in = out + (uint64_t)blocks * threads;
   if (which == 5 || which == 6) {
@@ -147,12 +147,14 @@ extern "C" __attribute__((visibility("default"))) int stk_microbench(stk_ctx* c,
       IPK(0) IPK(1) IPK(2) IPK(3) IPK(4) IPK(7) IPK(8) IPK(9) IPK(10) IPK(11) IPK(12) IPK(13)
 #undef IPK
       case 5:
-        if (c->is_stark) field_kernel<StarkField, 5><<<blocks, threads, 0, c->stream>>>(out, in, iters, StarkField());
-        else field_kernel<MontField, 5><<<blocks, threads, 0, c->stream>>>(out, in, iters, c->mont);
+        STK_TRY(stk_with_field(c, [&](auto f) {
+          field_kernel<decltype(f), 5><<<blocks, threads, 0, c->stream>>>(out, in, iters, f);
+        }));
         break;
       default:
-        if (c->is_stark) field_kernel<StarkField, 6><<<blocks, threads, 0, c->stream>>>(out, in, iters, StarkField());
-        else field_kernel<MontField, 6><<<blocks, threads, 0, c->stream>>>(out, in, iters, c->mont);
+        STK_TRY(stk_with_field(c, [&](auto f) {
+          field_kernel<decltype(f), 6><<<blocks, threads, 0, c->stream>>>(out, in, iters, f);
+        }));
         break;
     }
     STK_CUDA(c, cudaEventRecord(e1, c->stream));
@@ -182,14 +184,14 @@ static int run_variant(stk_ctx* c, int which, uint64_t iters, unsigned blocks, u
   return STK_OK;
 }
 
-extern "C" __attribute__((visibility("default"))) int stk_microbench_variant(stk_ctx* c, int variant, int which, uint64_t iters, float* ms,
-                                                                              double* ops, uint64_t* mismatches) {
+STK_API int stk_microbench_variant(stk_ctx* c, int variant, int which, uint64_t iters, float* ms, double* ops,
+                                   uint64_t* mismatches) {
   if (!c || !ms || !ops || !mismatches || (which != 5 && which != 6) || variant < 0 || variant > 3) return STK_EINVAL;
   if (!c->is_stark) return stk_fail(c, STK_EUNSUPPORTED, "the experimental multiply is for the STARK prime");
   const unsigned blocks = (unsigned)c->sm_count * 8, threads = 256;
   const uint64_t nthr = (uint64_t)blocks * threads;
   void* buf;
-  STK_TRY(stk_scratch(c, 2, (2 * nthr + 1024) * sizeof(fe), &buf));
+  STK_TRY(stk_scratch(c, kSlotStage, (2 * nthr + 1024) * sizeof(fe), &buf));
   fe* out = (fe*)buf;
   fe* ref = out + nthr;
   fe* in = ref + nthr;

@@ -18,6 +18,11 @@ fe stk_h_mul(stk_ctx* c, const fe& a, const fe& b) { return host::mulmod(a, b, c
 fe stk_h_pow(stk_ctx* c, const fe& a, uint64_t e) { return host::pow_u64(a, e, c->p); }
 fe stk_h_inv(stk_ctx* c, const fe& a) { return host::invmod(a, c->p); }
 fe stk_h_to_tw(stk_ctx* c, const fe& a) { return c->is_stark ? a : host::mulmod(a, c->mont.rone, c->p); }
+fe stk_h_one(stk_ctx* c) { return host::reduce(host::from_u64(1), c->p); }
+bool stk_h_primitive(stk_ctx* c, const fe& root, uint64_t n) {
+  const fe one = stk_h_one(c);
+  return fe_eq(stk_h_pow(c, root, n), one) && !fe_eq(stk_h_pow(c, root, n / 2), one);
+}
 
 void stk_stark_release(stk_ctx* c);  // stark.cu: per-context inverse tables
 
@@ -41,11 +46,19 @@ int stk_scratch(stk_ctx* c, int slot, uint64_t bytes, void** out) {
   return STK_OK;
 }
 
+int stk_stage(stk_ctx* c, int slot, uint64_t bytes, std::initializer_list<stk_upload> ups, void** out) {
+  STK_TRY(stk_scratch(c, slot, bytes, out));
+  for (const stk_upload& u : ups)
+    STK_CUDA(c, cudaMemcpyAsync((char*)*out + u.off, u.h, u.bytes, cudaMemcpyHostToDevice, c->stream));
+  STK_CUDA(c, cudaStreamSynchronize(c->stream));
+  return STK_OK;
+}
+
 // ------------------------------------------------------------------ context
 
-extern "C" __attribute__((visibility("default"))) int stk_version(void) { return 1; }
+STK_API int stk_version(void) { return 1; }
 
-extern "C" __attribute__((visibility("default"))) int stk_init(int device, stk_ctx** out) {
+STK_API int stk_init(int device, stk_ctx** out) {
   if (!out) return STK_EINVAL;
   *out = nullptr;
   int count = 0;
@@ -65,22 +78,22 @@ extern "C" __attribute__((visibility("default"))) int stk_init(int device, stk_c
   return STK_OK;
 }
 
-extern "C" __attribute__((visibility("default"))) void stk_destroy(stk_ctx* c) {
+STK_API void stk_destroy(stk_ctx* c) {
   if (!c) return;
   cudaSetDevice(c->device);
   cudaDeviceSynchronize();
   for (auto& t : c->tables) cudaFree(t.d);
   stk_stark_release(c);
-  for (int i = 0; i < stk_ctx::kScratchSlots; ++i) if (c->scratch[i]) cudaFree(c->scratch[i]);
+  for (int i = 0; i < kScratchSlots; ++i) if (c->scratch[i]) cudaFree(c->scratch[i]);
   for (int i = 0; i < 8; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
   for (int i = 0; i < 3; ++i) if (c->copy_streams[i]) cudaStreamDestroy(c->copy_streams[i]);
   if (c->own_stream) cudaStreamDestroy(c->own_stream);
   delete c;
 }
 
-extern "C" __attribute__((visibility("default"))) const char* stk_last_error(stk_ctx* c) { return c ? c->err.c_str() : "no context"; }
+STK_API const char* stk_last_error(stk_ctx* c) { return c ? c->err.c_str() : "no context"; }
 
-extern "C" __attribute__((visibility("default"))) int stk_set_stream(stk_ctx* c, void* s) {
+STK_API int stk_set_stream(stk_ctx* c, void* s) {
   if (!c) return STK_EINVAL;
   cudaStream_t next = s ? (cudaStream_t)s : c->own_stream;
   if (next != c->stream) {
@@ -92,13 +105,13 @@ extern "C" __attribute__((visibility("default"))) int stk_set_stream(stk_ctx* c,
   return STK_OK;
 }
 
-extern "C" __attribute__((visibility("default"))) int stk_sync(stk_ctx* c) {
+STK_API int stk_sync(stk_ctx* c) {
   if (!c) return STK_EINVAL;
   STK_CUDA(c, cudaStreamSynchronize(c->stream));
   return STK_OK;
 }
 
-extern "C" __attribute__((visibility("default"))) int stk_field_set(stk_ctx* c, const uint32_t p32[8]) {
+STK_API int stk_field_set(stk_ctx* c, const uint32_t p32[8]) {
   if (!c || !p32) return STK_EINVAL;
   fe p = stk_load_fe(p32);
   if (fe_eq(p, c->p)) return STK_OK;
@@ -124,44 +137,44 @@ extern "C" __attribute__((visibility("default"))) int stk_field_set(stk_ctx* c, 
 
 // ------------------------------------------------------------------ memory helpers
 
-extern "C" __attribute__((visibility("default"))) int stk_dev_alloc(stk_ctx* c, uint64_t bytes, void** d) {
+STK_API int stk_dev_alloc(stk_ctx* c, uint64_t bytes, void** d) {
   if (!c || !d) return STK_EINVAL;
   STK_CUDA(c, cudaMalloc(d, bytes ? bytes : 1));
   return STK_OK;
 }
-extern "C" __attribute__((visibility("default"))) int stk_dev_free(stk_ctx* c, void* d) {
+STK_API int stk_dev_free(stk_ctx* c, void* d) {
   if (!c) return STK_EINVAL;
   STK_CUDA(c, cudaStreamSynchronize(c->stream));
   STK_CUDA(c, cudaFree(d));
   return STK_OK;
 }
-extern "C" __attribute__((visibility("default"))) int stk_host_alloc(stk_ctx* c, uint64_t bytes, void** h) {
+STK_API int stk_host_alloc(stk_ctx* c, uint64_t bytes, void** h) {
   if (!c || !h) return STK_EINVAL;
   STK_CUDA(c, cudaHostAlloc(h, bytes ? bytes : 1, cudaHostAllocDefault));
   return STK_OK;
 }
-extern "C" __attribute__((visibility("default"))) int stk_host_free(stk_ctx* c, void* h) {
+STK_API int stk_host_free(stk_ctx* c, void* h) {
   if (!c) return STK_EINVAL;
   STK_CUDA(c, cudaFreeHost(h));
   return STK_OK;
 }
-extern "C" __attribute__((visibility("default"))) int stk_memcpy_h2d(stk_ctx* c, void* d, const void* h, uint64_t bytes) {
+STK_API int stk_memcpy_h2d(stk_ctx* c, void* d, const void* h, uint64_t bytes) {
   if (!c) return STK_EINVAL;
   STK_CUDA(c, cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, c->stream));
   return STK_OK;
 }
-extern "C" __attribute__((visibility("default"))) int stk_memcpy_d2h(stk_ctx* c, void* h, const void* d, uint64_t bytes) {
+STK_API int stk_memcpy_d2h(stk_ctx* c, void* h, const void* d, uint64_t bytes) {
   if (!c) return STK_EINVAL;
   STK_CUDA(c, cudaMemcpyAsync(h, d, bytes, cudaMemcpyDeviceToHost, c->stream));
   STK_CUDA(c, cudaStreamSynchronize(c->stream));
   return STK_OK;
 }
-extern "C" __attribute__((visibility("default"))) int stk_memcpy_d2d(stk_ctx* c, void* dd, const void* ds, uint64_t bytes) {
+STK_API int stk_memcpy_d2d(stk_ctx* c, void* dd, const void* ds, uint64_t bytes) {
   if (!c) return STK_EINVAL;
   STK_CUDA(c, cudaMemcpyAsync(dd, ds, bytes, cudaMemcpyDeviceToDevice, c->stream));
   return STK_OK;
 }
-extern "C" __attribute__((visibility("default"))) int stk_memset(stk_ctx* c, void* d, int value, uint64_t bytes) {
+STK_API int stk_memset(stk_ctx* c, void* d, int value, uint64_t bytes) {
   if (!c) return STK_EINVAL;
   STK_CUDA(c, cudaMemsetAsync(d, value, bytes, c->stream));
   return STK_OK;
@@ -202,18 +215,17 @@ int stk_get_table(stk_ctx* c, const fe& root, uint64_t n, const fe** d_table) {
   stk_table t;
   t.root = root; t.n = n; t.mont = !c->is_stark; t.d = nullptr;
   STK_CUDA(c, cudaMalloc(&t.d, std::max<uint64_t>(n, 1) * sizeof(fe)));
-  fe one = stk_h_to_tw(c, host::reduce(host::from_u64(1), c->p));
+  fe one = stk_h_to_tw(c, stk_h_one(c));
   STK_CUDA(c, cudaMemcpyAsync(t.d, &one, sizeof(fe), cudaMemcpyHostToDevice, c->stream));
-  fe wm = root;  // root^m, plain
-  for (uint64_t m = 1; m < n; m <<= 1) {
-    fe wm_tw = stk_h_to_tw(c, wm);
-    uint64_t cnt = std::min<uint64_t>(m, n - m);
-    unsigned blocks = (unsigned)((cnt + 255) / 256);
-    if (c->is_stark) twiddle_extend_kernel<StarkField><<<blocks, 256, 0, c->stream>>>(t.d, m, n, wm_tw, StarkField());
-    else twiddle_extend_kernel<MontField><<<blocks, 256, 0, c->stream>>>(t.d, m, n, wm_tw, c->mont);
-    wm = stk_h_mul(c, wm, wm);
-  }
-  STK_CUDA(c, cudaGetLastError());
+  STK_TRY(stk_with_field(c, [&](auto f) {
+    fe wm = root;  // root^m, plain
+    for (uint64_t m = 1; m < n; m <<= 1) {
+      uint64_t cnt = std::min<uint64_t>(m, n - m);
+      unsigned blocks = (unsigned)((cnt + 255) / 256);
+      twiddle_extend_kernel<<<blocks, 256, 0, c->stream>>>(t.d, m, n, stk_h_to_tw(c, wm), f);
+      wm = stk_h_mul(c, wm, wm);
+    }
+  }));
   c->tables.push_back(t);
   *d_table = t.d;
   return STK_OK;
@@ -242,9 +254,16 @@ int stk_get_table_strided(stk_ctx* c, const fe& root, uint64_t n, const fe** d_t
   return stk_get_table(c, root, n, d_table);
 }
 
-// ------------------------------------------------------------------ NTT plan
+int stk_get_table_shift(stk_ctx* c, const fe& root, uint64_t n, const fe** d_table, int* shift) {
+  uint64_t stride;
+  STK_TRY(stk_get_table_strided(c, root, n, d_table, &stride));
+  *shift = stk_ilog2(stride);
+  if ((1ull << *shift) == stride) return STK_OK;
+  *shift = 0;
+  return stk_get_table(c, root, n, d_table);
+}
 
-static int ilog2_u64(uint64_t x) { int l = 0; while ((1ull << l) < x) ++l; return l; }
+// ------------------------------------------------------------------ NTT plan
 
 // log2 radix of the STARK-prime rounds; radix-4 measured no faster: profiles/r01_ntt_radix_sweep.txt
 static const int kStarkRadix = 3;
@@ -274,7 +293,7 @@ static int build_plan(int n, uint64_t batch, std::vector<NttPass>& plan, int rma
     NttPass P;
     memset(&P, 0, sizeof P);
     P.n = n; P.n_tw = n; P.lo = 0; P.k = n;
-    P.logC = std::min(logT - n, ilog2_u64(batch));
+    P.logC = std::min(logT - n, stk_ilog2(batch));
     P.logT = P.k + P.logC;
     P.c_is_col = 1; P.cb = 0; P.nl = 0; P.sl = 0; P.sh = 0;
     P.final_pass = 1;
@@ -319,17 +338,14 @@ int stk_launch_pass_stark_cf(stk_ctx* c, cudaStream_t s, const NttPass& P);     
 int stk_launch_pass_stark_t11_cf(stk_ctx* c, cudaStream_t s, const NttPass& P);
 int stk_launch_pass_mont(stk_ctx* c, cudaStream_t s, const NttPass& P);       // run-time modulus, radix-4
 
-template <class F>
-static int launch_pass(stk_ctx* c, cudaStream_t s, const NttPass& P, const F&) {
-  if constexpr (F::kMontgomery) return stk_launch_pass_mont(c, s, P);
-  else {
+static int launch_pass(stk_ctx* c, cudaStream_t s, const NttPass& P) {
+  if (!c->is_stark) return stk_launch_pass_mont(c, s, P);
   const bool zs = P.zbit < 32 || (P.cshift && !P.in_virtual);  // expansion round / coset scaling on load
   const bool cf = !zs && P.cshift && (P.final_pass || P.cskip0);  // interleaved store / skipped r = 0 columns
   if (P.logT > 10)
     return zs ? stk_launch_pass_stark_t11_zs(c, s, P) : cf ? stk_launch_pass_stark_t11_cf(c, s, P) : stk_launch_pass_stark_t11(c, s, P);
   else
     return zs ? stk_launch_pass_stark_zs(c, s, P) : cf ? stk_launch_pass_stark_cf(c, s, P) : stk_launch_pass_stark(c, s, P);
-  }
 }
 
 // direct DFT for orders that are not a power of two >= 8 (_simple_ft, starks/fft.py:287-300)
@@ -350,6 +366,16 @@ __global__ void dft_generic_kernel(const fe* in, uint64_t n_in, uint64_t in_stri
   fe_store(out + col * out_stride + k, acc);
 }
 
+static int launch_dft(stk_ctx* c, cudaStream_t s, const fe* in, uint64_t n_in, uint64_t in_stride, fe* out,
+                      uint64_t out_stride, uint64_t n, uint64_t batch, const fe* W, uint64_t wstride, int do_scale,
+                      const fe& scale_tw) {
+  const unsigned blocks = (unsigned)((n * batch + 127) / 128);
+  return stk_with_field(c, [&](auto f) {
+    dft_generic_kernel<<<blocks, 128, 0, s>>>(in, n_in, in_stride, out, out_stride, n, batch, W, wstride, do_scale,
+                                              scale_tw, f);
+  });
+}
+
 // out[col][8K] = canonical(r0[col][K]): the residue-0 coset of an 8x extension is the input domain
 __global__ void r0_copy_kernel(const fe* __restrict__ r0, uint64_t r0_stride, fe* __restrict__ out, uint64_t out_stride,
                                uint64_t ns, uint64_t batch) {
@@ -360,6 +386,13 @@ __global__ void r0_copy_kernel(const fe* __restrict__ r0, uint64_t r0_stride, fe
   StarkField::canon(v.v);
   fe_store(out + col * out_stride + 8 * K, v);
 }
+
+// optional peer scatter of a transform's final pass (stk_ntt_dev_peer)
+struct stk_peer_leaf {
+  int g;                      // log2 of the rank count
+  uint32_t col0;              // global index of this rank's first column
+  const uint64_t* ptrs;       // nranks exchange buffers (columns_total x N/G elements each)
+};
 
 static int ntt_dev_on(stk_ctx* c, cudaStream_t s, int scratch_slot, const fe* d_in, uint64_t n_in, uint64_t in_stride,
                       fe* d_out, uint64_t out_stride, uint64_t n, uint64_t batch, const fe& root, int inverse,
@@ -384,13 +417,9 @@ static int ntt_dev_on(stk_ctx* c, cudaStream_t s, int scratch_slot, const fe* d_
   for (auto& e : c->ntt_consts)
     if (e.n == n && e.inverse == (inverse ? 1 : 0) && fe_eq(e.root, root)) { K = &e; break; }
   if (!K) {
-    fe one = host::reduce(host::from_u64(1), c->p);
-    fe rn = stk_h_pow(c, root, n);
-    if (!fe_eq(rn, one)) return stk_fail(c, STK_EINVAL, "root^n != 1: n is not the order of the root");
-    if (n % 2 == 0 && n > 1) {
-      fe rh = stk_h_pow(c, root, n / 2);
-      if (fe_eq(rh, one)) return stk_fail(c, STK_EINVAL, "root has order below n");
-    }
+    // odd orders (the direct DFT) are held to root^n == 1 only
+    if (n % 2 ? !fe_eq(stk_h_pow(c, root, n), stk_h_one(c)) : !stk_h_primitive(c, root, n))
+      return stk_fail(c, STK_EINVAL, "root is not a primitive n-th root of unity");
     stk_ntt_consts e;
     e.root = root; e.n = n; e.inverse = inverse ? 1 : 0;
     e.w = inverse ? stk_h_inv(c, root) : root;
@@ -400,28 +429,25 @@ static int ntt_dev_on(stk_ctx* c, cudaStream_t s, int scratch_slot, const fe* d_
     c->ntt_consts.push_back(e);
     K = &c->ntt_consts.back();
   }
-  const fe w = K->w;
+  const bool pow2 = (n & (n - 1)) == 0;
   if (K->table_gen != c->table_gen || !K->W) {
     const fe* Wt = nullptr;
     uint64_t ws = 1;
-    STK_TRY(stk_get_table_strided(c, w, n, &Wt, &ws));
-    for (auto& e : c->ntt_consts)  // K may have moved if the table build... it does not touch ntt_consts; re-find for safety
-      if (e.n == n && e.inverse == (inverse ? 1 : 0) && fe_eq(e.root, root)) { K = &e; break; }
+    if (pow2) {  // the pass kernels index by shift
+      int shift;
+      STK_TRY(stk_get_table_shift(c, K->w, n, &Wt, &shift));
+      ws = 1ull << shift;
+    } else {
+      STK_TRY(stk_get_table_strided(c, K->w, n, &Wt, &ws));
+    }
     K->W = Wt; K->wstride = ws; K->table_gen = c->table_gen;
   }
   const fe* W = K->W;
-  uint64_t wstride = K->wstride;
+  const uint64_t wstride = K->wstride;
   const int do_scale = inverse && scale;
   const fe scale_tw = K->scale_tw;
-  bool pow2 = (n & (n - 1)) == 0;
-  if (pow2 && (wstride & (wstride - 1))) {  // the pass kernels index by shift
-    STK_TRY(stk_get_table(c, w, n, &W));
-    wstride = 1;
-  }
   if (!pow2 || n < 8) {
     if (n > 4096) return stk_fail(c, STK_EUNSUPPORTED, "non power-of-two order above 4096");
-    uint64_t total = n * batch;
-    unsigned blocks = (unsigned)((total + 127) / 128);
     const fe* src = d_in;
     if ((const void*)d_in == (const void*)d_out) {  // every output reads the whole column
       void* tmp;
@@ -432,16 +458,9 @@ static int ntt_dev_on(stk_ctx* c, cudaStream_t s, int scratch_slot, const fe* d_
       src = (const fe*)tmp;
       in_stride = n_in;
     }
-    if (c->is_stark)
-      dft_generic_kernel<StarkField><<<blocks, 128, 0, s>>>(src, n_in, in_stride, d_out, out_stride, n, batch, W,
-                                                           wstride, do_scale, scale_tw, StarkField());
-    else
-      dft_generic_kernel<MontField><<<blocks, 128, 0, s>>>(src, n_in, in_stride, d_out, out_stride, n, batch, W,
-                                                          wstride, do_scale, scale_tw, c->mont);
-    STK_CUDA(c, cudaGetLastError());
-    return STK_OK;
+    return launch_dft(c, s, src, n_in, in_stride, d_out, out_stride, n, batch, W, wstride, do_scale, scale_tw);
   }
-  int logn = ilog2_u64(n);
+  int logn = stk_ilog2(n);
   std::vector<NttPass> plan;
   // Zero-padded forward transform (LDE, n_in <= N/8): eight coset transforms of order N/8 over
   // <w^8> as 8*batch virtual columns (ntt.cuh, cshift) -- the sub-transform's passes split its
@@ -471,7 +490,7 @@ static int ntt_dev_on(stk_ctx* c, cudaStream_t s, int scratch_slot, const fe* d_
         NttPass& P = plan[i];
         P.batch = (uint32_t)vb;
         P.W = W;
-        P.cs_shift = ilog2_u64(wstride);
+        P.cs_shift = stk_ilog2(wstride);
         P.tw_shift = P.cs_shift + 3;
         P.cshift = 3;
         P.in_virtual = i > 0;
@@ -481,7 +500,7 @@ static int ntt_dev_on(stk_ctx* c, cudaStream_t s, int scratch_slot, const fe* d_
         else { P.in = tmpc; P.in_col_stride = ns; P.n_in = (uint32_t)ns; }
         if (P.final_pass) { P.out = d_out; P.out_col_stride = out_stride; }
         else { P.out = tmpc; P.out_col_stride = ns; }
-        STK_TRY(launch_pass<StarkField>(c, s, P, StarkField()));
+        STK_TRY(launch_pass(c, s, P));
       }
       if (use_r0) {
         const uint64_t tot = ns * batch;
@@ -505,13 +524,13 @@ static int ntt_dev_on(stk_ctx* c, cudaStream_t s, int scratch_slot, const fe* d_
     NttPass& P = plan[i];
     P.batch = (uint32_t)batch;
     P.W = W;
-    P.tw_shift = ilog2_u64(wstride);
+    P.tw_shift = stk_ilog2(wstride);
     P.do_scale = (P.final_pass && do_scale) ? 1 : 0;
     P.scale = scale_tw;
     P.zbit = 32;
     if (i == 0 && n_in > 0 && n_in * 8 <= n && P.k >= 3 && c->is_stark) {
       // the top three levels only scale-and-copy: run them as the first (radix-8) round
-      P.zbit = ilog2_u64(n_in);             // 2^zbit >= n_in, and 2^zbit <= N/8
+      P.zbit = stk_ilog2(n_in);             // 2^zbit >= n_in, and 2^zbit <= N/8
       if (P.r[0] != 3) {                    // remainder round goes last in this pass
         int rem = P.r[0];
         for (int q = 0; q + 1 < P.nrounds; ++q) P.r[q] = P.r[q + 1];
@@ -543,33 +562,35 @@ static int ntt_dev_on(stk_ctx* c, cudaStream_t s, int scratch_slot, const fe* d_
         for (int r2 = 0; r2 < (1 << peer->g); ++r2) P.peer_out[r2] = (fe*)(uintptr_t)peer->ptrs[r2];
       }
     }
-    if (c->is_stark) STK_TRY(launch_pass<StarkField>(c, s, P, StarkField()));
-    else STK_TRY(launch_pass<MontField>(c, s, P, c->mont));
+    STK_TRY(launch_pass(c, s, P));
   }
   return STK_OK;
 }
 
 int stk_ntt_dev_peer(stk_ctx* c, const fe* d_in, uint64_t n_in, uint64_t in_stride, uint64_t n, uint64_t batch,
-                     const fe& root, const stk_peer_leaf& peer) {
+                     const fe& root, uint64_t nranks, uint64_t col_base, const uint64_t* ptrs) {
+  const stk_peer_leaf peer = {stk_ilog2(nranks), (uint32_t)col_base, ptrs};
   // d_out is never written in peer mode; any distinct non-null pointer keeps the in-place logic off
-  return ntt_dev_on(c, c->stream, 0, d_in, n_in, in_stride, (fe*)(uintptr_t)16, n, n, batch, root, 0, 0, &peer);
+  return ntt_dev_on(c, c->stream, kSlotNtt, d_in, n_in, in_stride, (fe*)(uintptr_t)16, n, n, batch, root, 0, 0,
+                    &peer);
 }
 
 // Forward transform of coefficient rows whose values on the order-n/8 subgroup are already known
 // (r0: the trace an 8x low-degree extension started from): see NttPass::cskip0.
 int stk_ntt_dev_r0(stk_ctx* c, const fe* d_in, uint64_t n_in, uint64_t in_stride, fe* d_out, uint64_t out_stride,
                    uint64_t n, uint64_t batch, const fe& root, const fe* r0, uint64_t r0_stride) {
-  return ntt_dev_on(c, c->stream, 0, d_in, n_in, in_stride, d_out, out_stride, n, batch, root, 0, 0, nullptr, r0,
-                    r0_stride);
+  return ntt_dev_on(c, c->stream, kSlotNtt, d_in, n_in, in_stride, d_out, out_stride, n, batch, root, 0, 0, nullptr,
+                    r0, r0_stride);
 }
 
 int stk_ntt_dev(stk_ctx* c, const fe* d_in, uint64_t n_in, uint64_t in_stride, fe* d_out, uint64_t out_stride,
                 uint64_t n, uint64_t batch, const fe& root, int inverse, int scale) {
-  return ntt_dev_on(c, c->stream, 0, d_in, n_in, in_stride, d_out, out_stride, n, batch, root, inverse, scale);
+  return ntt_dev_on(c, c->stream, kSlotNtt, d_in, n_in, in_stride, d_out, out_stride, n, batch, root, inverse,
+                    scale);
 }
 
-extern "C" __attribute__((visibility("default"))) int stk_ntt(stk_ctx* c, const uint32_t* d_in, uint64_t n_in, uint64_t in_stride, uint32_t* d_out,
-                       uint64_t out_stride, uint64_t n, uint64_t batch, const uint32_t root[8], int inverse) {
+STK_API int stk_ntt(stk_ctx* c, const uint32_t* d_in, uint64_t n_in, uint64_t in_stride, uint32_t* d_out,
+                    uint64_t out_stride, uint64_t n, uint64_t batch, const uint32_t root[8], int inverse) {
   if (!c || !d_out || !root || (!d_in && n_in)) return STK_EINVAL;
   return stk_ntt_dev(c, (const fe*)d_in, n_in, in_stride, (fe*)d_out, out_stride, n, batch, stk_load_fe(root),
                      inverse, 1);
@@ -577,40 +598,30 @@ extern "C" __attribute__((visibility("default"))) int stk_ntt(stk_ctx* c, const 
 
 // _simple_ft (starks/fft.py:287-300) as its own entry point: the direct O(n^2) sum for ANY order
 // n <= 4096 (stk_ntt routes orders that are not a power of two >= 8 here on its own).
-extern "C" __attribute__((visibility("default"))) int stk_dft_generic(stk_ctx* c, const uint32_t* d_in, uint64_t n_in,
-                                                                       uint64_t in_stride, uint32_t* d_out,
-                                                                       uint64_t out_stride, uint64_t n, uint64_t batch,
-                                                                       const uint32_t root[8], int inverse) {
+STK_API int stk_dft_generic(stk_ctx* c, const uint32_t* d_in, uint64_t n_in, uint64_t in_stride, uint32_t* d_out,
+                            uint64_t out_stride, uint64_t n, uint64_t batch, const uint32_t root[8], int inverse) {
   if (!c || !d_out || !root || (!d_in && n_in)) return STK_EINVAL;
   if (n == 0 || batch == 0) return STK_OK;
   if (n_in > n) return stk_fail(c, STK_EINDEX, "input length exceeds the order of the root");
   if (n > 4096) return stk_fail(c, STK_EUNSUPPORTED, "direct DFT is limited to orders <= 4096");
   if ((const void*)d_in == (const void*)d_out) return stk_fail(c, STK_EINVAL, "direct DFT works out of place");
   fe r = host::reduce(stk_load_fe(root), c->p);
-  fe one = host::reduce(host::from_u64(1), c->p);
-  if (!fe_eq(stk_h_pow(c, r, n), one)) return stk_fail(c, STK_EINVAL, "root^n != 1");
+  if (!fe_eq(stk_h_pow(c, r, n), stk_h_one(c))) return stk_fail(c, STK_EINVAL, "root^n != 1");
   fe w = inverse ? stk_h_inv(c, r) : r;
   const fe* W = nullptr;
   uint64_t ws = 1;
   STK_TRY(stk_get_table_strided(c, w, n, &W, &ws));
   fe scale_tw = fe_zero();
   if (inverse) scale_tw = stk_h_to_tw(c, stk_h_inv(c, host::reduce(host::from_u64(n), c->p)));
-  unsigned blocks = (unsigned)((n * batch + 127) / 128);
-  if (c->is_stark)
-    dft_generic_kernel<StarkField><<<blocks, 128, 0, c->stream>>>((const fe*)d_in, n_in, in_stride, (fe*)d_out, out_stride,
-                                                                  n, batch, W, ws, inverse ? 1 : 0, scale_tw, StarkField());
-  else
-    dft_generic_kernel<MontField><<<blocks, 128, 0, c->stream>>>((const fe*)d_in, n_in, in_stride, (fe*)d_out, out_stride,
-                                                                 n, batch, W, ws, inverse ? 1 : 0, scale_tw, c->mont);
-  STK_CUDA(c, cudaGetLastError());
-  return STK_OK;
+  return launch_dft(c, c->stream, (const fe*)d_in, n_in, in_stride, (fe*)d_out, out_stride, n, batch, W, ws,
+                    inverse ? 1 : 0, scale_tw);
 }
 
 // Host buffers: columns stream through three device slots, each with its own stream, so that
 // the H2D copy of chunk i+1, the transform of chunk i and the D2H copy of chunk i-1 overlap
 // (PCIe is full duplex; the transform itself is ~5x faster than either copy).
-extern "C" __attribute__((visibility("default"))) int stk_ntt_host(stk_ctx* c, const uint32_t* h_in, uint64_t n_in, uint64_t in_stride, uint32_t* h_out,
-                            uint64_t out_stride, uint64_t n, uint64_t batch, const uint32_t root[8], int inverse) {
+STK_API int stk_ntt_host(stk_ctx* c, const uint32_t* h_in, uint64_t n_in, uint64_t in_stride, uint32_t* h_out,
+                         uint64_t out_stride, uint64_t n, uint64_t batch, const uint32_t root[8], int inverse) {
   if (!c || !h_out || !root || (!h_in && n_in)) return STK_EINVAL;
   if (n_in > n) return stk_fail(c, STK_EINDEX, "input length exceeds the order of the root");
   if (n == 0 || batch == 0) return STK_OK;
@@ -622,7 +633,7 @@ extern "C" __attribute__((visibility("default"))) int stk_ntt_host(stk_ctx* c, c
   // slot buffers: in (n_in per column, packed) and out (n per column)
   void* bufs;
   const uint64_t in_b = chunk * std::max<uint64_t>(n_in, 1) * sizeof(fe), out_b = chunk * col_bytes;
-  STK_TRY(stk_scratch(c, 7, kSlots * (in_b + out_b), &bufs));
+  STK_TRY(stk_scratch(c, kSlotHostNttBufs, kSlots * (in_b + out_b), &bufs));
   char* base = (char*)bufs;
   fe* din[kSlots];
   fe* dout[kSlots];
@@ -636,7 +647,7 @@ extern "C" __attribute__((visibility("default"))) int stk_ntt_host(stk_ctx* c, c
     fe w = inverse ? stk_h_inv(c, r) : r;
     STK_TRY(stk_get_table(c, w, n, &W));
     void* t;
-    for (int i = 0; i < kSlots; ++i) STK_TRY(stk_scratch(c, 4 + i, chunk * col_bytes, &t));
+    for (int i = 0; i < kSlots; ++i) STK_TRY(stk_scratch(c, kSlotHostNtt + i, chunk * col_bytes, &t));
     STK_CUDA(c, cudaStreamSynchronize(c->stream));
   }
   int slot = 0;
@@ -651,7 +662,7 @@ extern "C" __attribute__((visibility("default"))) int stk_ntt_host(stk_ctx* c, c
         STK_CUDA(c, cudaMemcpy2DAsync(din[slot], n_in * sizeof(fe), h_in + b0 * in_stride * 8,
                                       in_stride * sizeof(fe), n_in * sizeof(fe), nb, cudaMemcpyHostToDevice, s));
     }
-    STK_TRY(ntt_dev_on(c, s, 4 + slot, din[slot], n_in, n_in, dout[slot], n, n, nb, r, inverse, 1));
+    STK_TRY(ntt_dev_on(c, s, kSlotHostNtt + slot, din[slot], n_in, n_in, dout[slot], n, n, nb, r, inverse, 1));
     if (out_stride == n)
       STK_CUDA(c, cudaMemcpyAsync(h_out + b0 * out_stride * 8, dout[slot], nb * col_bytes, cudaMemcpyDeviceToHost, s));
     else
@@ -680,14 +691,13 @@ static int dist_phase_impl(stk_ctx* c, int phase, const uint32_t* d_in, uint32_t
   if ((local_n & (local_n - 1)) || (nranks & (nranks - 1)) || nranks < 2 || rank >= nranks || nranks > 8)
     return stk_fail(c, STK_EINVAL, "local length and rank count must be powers of two (2..8 ranks)");
   if (phase != 0 && phase != 1) return STK_EINVAL;
-  const int nloc = ilog2_u64(local_n), g = ilog2_u64(nranks), n = nloc + g;
+  const int nloc = stk_ilog2(local_n), g = stk_ilog2(nranks), n = nloc + g;
   if (n > 30 || nloc < 3) return stk_fail(c, STK_EUNSUPPORTED, "distributed transform needs 2^3 <= local length and N <= 2^30");
   if (phase == 0 && d_in != d_out) return stk_fail(c, STK_EINVAL, "phase 0 works in place");
   if (phase == 1 && (const void*)d_in == (const void*)d_out) return stk_fail(c, STK_EINVAL, "phase 1 works out of place");
   fe r = stk_load_fe(root);
   const uint64_t N = local_n * nranks;
-  fe one = host::reduce(host::from_u64(1), c->p);
-  if (!fe_eq(stk_h_pow(c, r, N), one) || fe_eq(stk_h_pow(c, r, N / 2), one))
+  if (!stk_h_primitive(c, r, N))
     return stk_fail(c, STK_EINVAL, "root is not a primitive (G*L)-th root of unity");
   fe w = inverse ? stk_h_inv(c, r) : r;
   const fe* W = nullptr;
@@ -735,15 +745,14 @@ static int dist_phase_impl(stk_ctx* c, int phase, const uint32_t* d_in, uint32_t
     P.out = (fe*)d_out; P.out_col_stride = stride;
     P.do_scale = (P.final_pass && do_scale) ? 1 : 0;
     P.scale = scale_tw;
-    if (c->is_stark) STK_TRY(launch_pass<StarkField>(c, c->stream, P, StarkField()));
-    else STK_TRY(launch_pass<MontField>(c, c->stream, P, c->mont));
+    STK_TRY(launch_pass(c, c->stream, P));
   }
   return STK_OK;
 }
 
-extern "C" __attribute__((visibility("default"))) int stk_ntt_dist_phase(
-    stk_ctx* c, int phase, const uint32_t* d_in, uint32_t* d_out, uint64_t local_n, uint64_t batch, uint64_t stride,
-    const uint32_t root[8], uint64_t nranks, uint64_t rank, int inverse) {
+STK_API int stk_ntt_dist_phase(stk_ctx* c, int phase, const uint32_t* d_in, uint32_t* d_out, uint64_t local_n,
+                               uint64_t batch, uint64_t stride, const uint32_t root[8], uint64_t nranks, uint64_t rank,
+                               int inverse) {
   if (phase == 2)  // phase 1 on the untransposed exchange layout [source rank][m]
     return dist_phase_impl(c, 1, d_in, d_out, local_n, batch, stride, root, nranks, rank, inverse, nullptr, 1);
   return dist_phase_impl(c, phase, d_in, d_out, local_n, batch, stride, root, nranks, rank, inverse, nullptr, 0);
@@ -753,9 +762,8 @@ extern "C" __attribute__((visibility("default"))) int stk_ntt_dist_phase(
 // owning rank's exchange buffer over NVLink (peer_ptrs[r] = rank r's buffer mapped into this
 // process, e.g. torch symmetric memory), so no separate all-to-all or transpose pass runs.
 // The caller orders it with a cross-rank barrier before stk_ntt_dist_phase(phase = 2).
-extern "C" __attribute__((visibility("default"))) int stk_ntt_dist_phase0_p2p(
-    stk_ctx* c, uint32_t* d_inout, uint64_t local_n, const uint32_t root[8], uint64_t nranks, uint64_t rank,
-    int inverse, const uint64_t* peer_ptrs) {
+STK_API int stk_ntt_dist_phase0_p2p(stk_ctx* c, uint32_t* d_inout, uint64_t local_n, const uint32_t root[8],
+                                    uint64_t nranks, uint64_t rank, int inverse, const uint64_t* peer_ptrs) {
   if (!peer_ptrs) return STK_EINVAL;
   return dist_phase_impl(c, 0, d_inout, d_inout, local_n, 1, local_n, root, nranks, rank, inverse, peer_ptrs, 0);
 }
@@ -773,23 +781,22 @@ __global__ void vec_op_kernel(int op, const fe* a, const fe* b, fe* out, uint64_
   fe_store(out + i, r);
 }
 
-extern "C" __attribute__((visibility("default"))) int stk_vec_op(stk_ctx* c, int op, const uint32_t* d_a, const uint32_t* d_b, uint32_t* d_out, uint64_t n) {
+STK_API int stk_vec_op(stk_ctx* c, int op, const uint32_t* d_a, const uint32_t* d_b, uint32_t* d_out, uint64_t n) {
   if (!c || op < 0 || op > 2) return STK_EINVAL;
   if (!n) return STK_OK;
   unsigned blocks = (unsigned)((n + 255) / 256);
-  if (c->is_stark) vec_op_kernel<StarkField><<<blocks, 256, 0, c->stream>>>(op, (const fe*)d_a, (const fe*)d_b, (fe*)d_out, n, StarkField());
-  else vec_op_kernel<MontField><<<blocks, 256, 0, c->stream>>>(op, (const fe*)d_a, (const fe*)d_b, (fe*)d_out, n, c->mont);
-  STK_CUDA(c, cudaGetLastError());
-  return STK_OK;
+  return stk_with_field(c, [&](auto f) {
+    vec_op_kernel<<<blocks, 256, 0, c->stream>>>(op, (const fe*)d_a, (const fe*)d_b, (fe*)d_out, n, f);
+  });
 }
 
-extern "C" __attribute__((visibility("default"))) int stk_mul_polys(stk_ctx* c, const uint32_t* d_a, uint64_t na, const uint32_t* d_b, uint64_t nb,
-                             uint32_t* d_out, uint64_t n, const uint32_t root[8]) {
+STK_API int stk_mul_polys(stk_ctx* c, const uint32_t* d_a, uint64_t na, const uint32_t* d_b, uint64_t nb,
+                          uint32_t* d_out, uint64_t n, const uint32_t root[8]) {
   if (!c || !d_out || !root) return STK_EINVAL;
   if (na > n || nb > n) return stk_fail(c, STK_EINDEX, "operand longer than the order of the root");
   fe r = stk_load_fe(root);
   void* t;
-  STK_TRY(stk_scratch(c, 2, 2 * n * sizeof(fe), &t));
+  STK_TRY(stk_scratch(c, kSlotStage, 2 * n * sizeof(fe), &t));
   fe* x1 = (fe*)t;
   fe* x2 = x1 + n;
   STK_TRY(stk_ntt_dev(c, (const fe*)d_a, na, na, x1, n, n, 1, r, 0, 0));
@@ -806,7 +813,7 @@ __global__ void from_tw_kernel(const fe* W, fe* out, uint64_t n, const F f) {
   if (i < n) fe_store(out + i, f.from_tw(fe_load(W + i)));
 }
 
-extern "C" __attribute__((visibility("default"))) int stk_power_cycle(stk_ctx* c, const uint32_t r32[8], uint64_t n, uint32_t* d_out) {
+STK_API int stk_power_cycle(stk_ctx* c, const uint32_t r32[8], uint64_t n, uint32_t* d_out) {
   if (!c || !r32 || !d_out) return STK_EINVAL;
   if (!n) return STK_OK;
   const fe* W;

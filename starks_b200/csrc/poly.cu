@@ -15,11 +15,6 @@
 
 using namespace stk;
 
-// scratch slots of this file (ctx.h): the transform route's evaluations (mul_low), divmod's
-// temporaries, and the two buffers of composition and multivariate evaluation.  mul_low writes
-// kSlotEvals, so nothing that outlives a mul_low call may live there.
-static const int kSlotEvals = 12, kSlotDiv = 13, kSlotComp = 14, kSlotComp2 = 15;
-
 static uint64_t pow2_at_least(uint64_t x) {
   uint64_t L = 1;
   while (L < x) L <<= 1;
@@ -43,7 +38,7 @@ struct PolyRoots {
 
 static PolyRoots poly_roots(stk_ctx* c) {
   PolyRoots R;
-  const fe p = c->p, one = host::reduce(host::from_u64(1), p);
+  const fe p = c->p, one = stk_h_one(c);
   R.w[0] = one;
   fe pm1;
   sub8(pm1.v, p.v, one.v);
@@ -132,7 +127,7 @@ static int mul_low(stk_ctx* c, const PolyRoots& R, const fe* a, uint64_t na, con
     return STK_OK;
   }
   void* t;
-  STK_TRY(stk_scratch(c, kSlotEvals, 2 * L * sizeof(fe), &t));
+  STK_TRY(stk_scratch(c, kSlotPolyEvals, 2 * L * sizeof(fe), &t));
   fe* A = (fe*)t;
   fe* B = A + L;
   STK_TRY(stk_ntt_dev(c, a, na, na, A, L, L, 1, R.w[s], 0, 0));
@@ -146,8 +141,8 @@ static int mul_low(stk_ctx* c, const PolyRoots& R, const fe* a, uint64_t na, con
   return STK_OK;
 }
 
-extern "C" __attribute__((visibility("default"))) int stk_poly_mul(stk_ctx* c, const uint32_t* d_a, uint64_t na,
-                                                                    const uint32_t* d_b, uint64_t nb, uint32_t* d_out) {
+STK_API int stk_poly_mul(stk_ctx* c, const uint32_t* d_a, uint64_t na, const uint32_t* d_b, uint64_t nb,
+                         uint32_t* d_out) {
   if (!c) return STK_EINVAL;
   if (!na || !nb) return STK_OK;
   if (!d_a || !d_b || !d_out) return stk_fail(c, STK_EINVAL, "null pointer");
@@ -158,9 +153,8 @@ extern "C" __attribute__((visibility("default"))) int stk_poly_mul(stk_ctx* c, c
   return mul_low(c, R, (const fe*)d_a, na, (const fe*)d_b, nb, (fe*)d_out, m);
 }
 
-extern "C" __attribute__((visibility("default"))) int stk_poly_divmod(stk_ctx* c, const uint32_t* d_a, uint64_t na,
-                                                                       const uint32_t* d_b, uint64_t nb, uint32_t* d_q,
-                                                                       uint32_t* d_r) {
+STK_API int stk_poly_divmod(stk_ctx* c, const uint32_t* d_a, uint64_t na, const uint32_t* d_b, uint64_t nb,
+                            uint32_t* d_q, uint32_t* d_r) {
   if (!c) return STK_EINVAL;
   if (nb == 0 || !d_b) return stk_fail(c, STK_EINVAL, "the divisor has no coefficients");
   const uint64_t k = na >= nb ? na - nb + 1 : 0, nr = nb - 1;
@@ -172,9 +166,8 @@ extern "C" __attribute__((visibility("default"))) int stk_poly_divmod(stk_ctx* c
   STK_CUDA(c, cudaMemcpyAsync(&lead, d_b + 8 * (nb - 1), sizeof(fe), cudaMemcpyDeviceToHost, c->stream));
   STK_CUDA(c, cudaStreamSynchronize(c->stream));
   lead = host::reduce(lead, c->p);
-  const fe one = host::reduce(host::from_u64(1), c->p);
   const fe inv = stk_h_inv(c, lead);
-  if (!fe_eq(stk_h_mul(c, lead, inv), one))
+  if (!fe_eq(stk_h_mul(c, lead, inv), stk_h_one(c)))
     return stk_fail(c, STK_EINVAL, "the divisor's leading coefficient is zero (or not invertible mod p)");
   const fe* a = (const fe*)d_a;
   const fe* b = (const fe*)d_b;
@@ -187,7 +180,7 @@ extern "C" __attribute__((visibility("default"))) int stk_poly_divmod(stk_ctx* c
   // f = rev(b) mod X^k, g = f^-1 mod X^k, ra = rev(a) mod X^k; t holds a product of length <= k
   const uint64_t nf = std::min(nb, k);
   void* scr;
-  STK_TRY(stk_scratch(c, kSlotDiv, (nf + 3 * k) * sizeof(fe), &scr));
+  STK_TRY(stk_scratch(c, kSlotPolyDiv, (nf + 3 * k) * sizeof(fe), &scr));
   fe* f = (fe*)scr;
   fe* g = f + nf;
   fe* ra = g + k;
@@ -201,14 +194,14 @@ extern "C" __attribute__((visibility("default"))) int stk_poly_divmod(stk_ctx* c
     STK_TRY(check_length(c, s));
     if (s <= R.smax) {
       void* e;
-      STK_TRY(stk_scratch(c, kSlotEvals, 2 * L * sizeof(fe), &e));
+      STK_TRY(stk_scratch(c, kSlotPolyEvals, 2 * L * sizeof(fe), &e));
       fe* Fv = (fe*)e;
       fe* Gv = Fv + L;
       STK_TRY(stk_ntt_dev(c, f, nf2, nf2, Fv, L, L, 1, R.w[s], 0, 0));
       STK_TRY(stk_ntt_dev(c, g, l, l, Gv, L, L, 1, R.w[s], 0, 0));
-      if (c->is_stark) newton_recip_kernel<StarkField><<<blocks_for(L, 256), 256, 0, c->stream>>>(Fv, Gv, L, StarkField());
-      else newton_recip_kernel<MontField><<<blocks_for(L, 256), 256, 0, c->stream>>>(Fv, Gv, L, c->mont);
-      STK_CUDA(c, cudaGetLastError());
+      STK_TRY(stk_with_field(c, [&](auto f) {
+        newton_recip_kernel<<<blocks_for(L, 256), 256, 0, c->stream>>>(Fv, Gv, L, f);
+      }));
       STK_TRY(stk_ntt_dev(c, Gv, L, L, Fv, L, L, 1, R.w[s], 1, 1));
       STK_CUDA(c, cudaMemcpyAsync(g + l, Fv + l, (l2 - l) * sizeof(fe), cudaMemcpyDeviceToDevice, c->stream));
     } else {
@@ -289,16 +282,10 @@ __global__ void compose_combine_kernel(const fe* __restrict__ prev, uint64_t np,
   fe_store(out + idx, v);
 }
 
-#define POLY_LAUNCH(c, kernel, n, ...)                                                                          \
-  do {                                                                                                          \
-    if ((c)->is_stark) kernel<StarkField><<<blocks_for((n), 256), 256, 0, (c)->stream>>>(__VA_ARGS__, StarkField()); \
-    else kernel<MontField><<<blocks_for((n), 256), 256, 0, (c)->stream>>>(__VA_ARGS__, (c)->mont);                 \
-    STK_CUDA((c), cudaGetLastError());                                                                          \
-  } while (0)
-
 // `batch` transforms of length n (columns at in_stride, n_in coefficients each, zero-padded) into
 // out at stride n; the inverse is scaled.  Multi-pass transforms take at most 65535 columns per
-// launch (ntt.cuh), so large batches go in groups.
+// launch (ntt.cuh), so large batches go in groups: stk_ntt_dev only groups transforms longer than
+// 2048, and a run-time modulus already takes two passes at 2048 (1024-element tiles).
 static int ntt_cols(stk_ctx* c, const fe* in, uint64_t n_in, uint64_t in_stride, fe* out, uint64_t n, uint64_t batch,
                     const fe& root, int inverse) {
   for (uint64_t b0 = 0; b0 < batch; b0 += 32768) {
@@ -321,8 +308,9 @@ static int compose_general(stk_ctx* c, const fe* a, uint64_t na, const fe* b, ui
   const uint64_t d = nb - 1, N = pow2_at_least(na);
   const int levels = __builtin_ctzll(N);
   if (levels == 1) {
-    POLY_LAUNCH(c, compose_level0_kernel, nb, a, na, b, nb, out, 1);
-    return STK_OK;
+    return stk_with_field(c, [&](auto f) {
+      compose_level0_kernel<<<blocks_for(nb, 256), 256, 0, c->stream>>>(a, na, b, nb, out, 1, f);
+    });
   }
   auto chunk = [&](int j) -> uint64_t { return j + 1 == levels ? nout : ((2ull << j) - 1) * d + 1; };
   uint64_t cur_max = (N / 2) * nb, t_max = 0, b_max = 2 * d + 1;
@@ -335,14 +323,16 @@ static int compose_general(stk_ctx* c, const fe* a, uint64_t na, const fe* b, ui
   }
   void* s1;
   void* s2;
-  STK_TRY(stk_scratch(c, kSlotComp, 2 * cur_max * sizeof(fe), &s1));
-  STK_TRY(stk_scratch(c, kSlotComp2, (t_max + 2 * b_max) * sizeof(fe), &s2));
+  STK_TRY(stk_scratch(c, kSlotPolyA, 2 * cur_max * sizeof(fe), &s1));
+  STK_TRY(stk_scratch(c, kSlotPolyB, (t_max + 2 * b_max) * sizeof(fe), &s2));
   fe* cur = (fe*)s1;
   fe* nxt = cur + cur_max;
   fe* T = (fe*)s2;
   fe* Bp = T + t_max;   // coefficients of b^(2^j)
   fe* Bv = Bp + b_max;  // its transform (product route: the next power)
-  POLY_LAUNCH(c, compose_level0_kernel, (N / 2) * nb, a, na, b, nb, cur, N / 2);
+  STK_TRY(stk_with_field(c, [&](auto f) {
+    compose_level0_kernel<<<blocks_for((N / 2) * nb, 256), 256, 0, c->stream>>>(a, na, b, nb, cur, N / 2, f);
+  }));
   STK_TRY(mul_low(c, R, b, nb, b, nb, Bp, 2 * d + 1));
   uint64_t np = nb;
   for (int j = 1; j < levels; ++j) {
@@ -356,7 +346,9 @@ static int compose_general(stk_ctx* c, const fe* a, uint64_t na, const fe* b, ui
       ts = L;
       STK_TRY(ntt_cols(c, cur + np, np, 2 * np, T, L, batch, R.w[s], 0));
       STK_TRY(stk_ntt_dev(c, Bp, nbp, nbp, Bv, Lb, Lb, 1, R.w[sb], 0, 0));
-      POLY_LAUNCH(c, mul_bcast_kernel, batch * L, T, L, batch * L, Bv, Lb / L);
+      STK_TRY(stk_with_field(c, [&](auto f) {
+        mul_bcast_kernel<<<blocks_for(batch * L, 256), 256, 0, c->stream>>>(T, L, batch * L, Bv, Lb / L, f);
+      }));
       STK_TRY(ntt_cols(c, T, L, L, T, L, batch, R.w[s], 1));
       if (!top) {
         STK_TRY(stk_vec_op(c, 2, (const uint32_t*)Bv, (const uint32_t*)Bv, (uint32_t*)Bv, Lb));
@@ -369,16 +361,17 @@ static int compose_general(stk_ctx* c, const fe* a, uint64_t na, const fe* b, ui
         std::swap(Bp, Bv);
       }
     }
-    POLY_LAUNCH(c, compose_combine_kernel, batch * nn, cur, np, T, ts, dst, nn, batch);
+    STK_TRY(stk_with_field(c, [&](auto f) {
+      compose_combine_kernel<<<blocks_for(batch * nn, 256), 256, 0, c->stream>>>(cur, np, T, ts, dst, nn, batch, f);
+    }));
     std::swap(cur, nxt);
     np = nn;
   }
   return STK_OK;
 }
 
-extern "C" __attribute__((visibility("default"))) int stk_poly_compose(stk_ctx* c, const uint32_t* d_a, uint64_t na,
-                                                                        const uint32_t* d_b, uint64_t nb,
-                                                                        uint32_t* d_out) {
+STK_API int stk_poly_compose(stk_ctx* c, const uint32_t* d_a, uint64_t na, const uint32_t* d_b, uint64_t nb,
+                             uint32_t* d_out) {
   if (!c) return STK_EINVAL;
   if (nb < 2) return stk_fail(c, STK_EINVAL, "the inner polynomial needs at least two coefficients");
   if (!na) return STK_OK;
@@ -400,8 +393,9 @@ extern "C" __attribute__((visibility("default"))) int stk_poly_compose(stk_ctx* 
     if (fe_eq(host::reduce(b01[0], c->p), fe_zero())) {
       const fe alpha_tw = stk_h_to_tw(c, host::reduce(b01[1], c->p));
       const uint64_t threads = (na + kScaleChunk - 1) / kScaleChunk;
-      POLY_LAUNCH(c, scale_powers_kernel, threads, a, na, alpha_tw, (fe*)d_out);
-      return STK_OK;
+      return stk_with_field(c, [&](auto f) {
+        scale_powers_kernel<<<blocks_for(threads, 256), 256, 0, c->stream>>>(a, na, alpha_tw, (fe*)d_out, f);
+      });
     }
   }
   return compose_general(c, a, na, b, nb, (fe*)d_out, m);
@@ -486,10 +480,10 @@ static int multivar_products(stk_ctx* c, const fe* polys, const uint64_t* lens, 
   return STK_OK;
 }
 
-extern "C" __attribute__((visibility("default"))) int stk_poly_eval_multivar(
-    stk_ctx* c, const uint32_t* d_polys, const uint64_t* h_lens, uint64_t in_stride, uint64_t width,
-    const uint32_t* h_mono_out, const uint32_t* h_mono_coeffs, const uint32_t* h_mono_exps, uint64_t nmono,
-    uint64_t nout, uint32_t* d_out, uint64_t out_len) {
+STK_API int stk_poly_eval_multivar(stk_ctx* c, const uint32_t* d_polys, const uint64_t* h_lens, uint64_t in_stride,
+                                   uint64_t width, const uint32_t* h_mono_out, const uint32_t* h_mono_coeffs,
+                                   const uint32_t* h_mono_exps, uint64_t nmono, uint64_t nout, uint32_t* d_out,
+                                   uint64_t out_len) {
   if (!c) return STK_EINVAL;
   if (width == 0 || width > 12) return stk_fail(c, STK_EUNSUPPORTED, "width must be in 1..12");
   if (!h_lens || (nmono && (!h_mono_out || !h_mono_coeffs || !h_mono_exps)))
@@ -539,12 +533,11 @@ extern "C" __attribute__((visibility("default"))) int stk_poly_eval_multivar(
   if (s > R.smax) {
     std::vector<fe> coeffs(nmono ? nmono : 1);
     for (uint64_t m = 0; m < nmono; ++m) coeffs[m] = host::reduce(stk_load_fe(h_mono_coeffs + 8 * m), c->p);
+    const uint64_t coeff_bytes = coeffs.size() * sizeof(fe);
     void* w;
     void* cf;
-    STK_TRY(stk_scratch(c, kSlotComp, 3 * out_len * sizeof(fe), &w));
-    STK_TRY(stk_scratch(c, kSlotComp2, coeffs.size() * sizeof(fe), &cf));
-    STK_CUDA(c, cudaMemcpyAsync(cf, coeffs.data(), coeffs.size() * sizeof(fe), cudaMemcpyHostToDevice, c->stream));
-    STK_CUDA(c, cudaStreamSynchronize(c->stream));  // coeffs is a stack-owned staging buffer
+    STK_TRY(stk_scratch(c, kSlotPolyA, 3 * out_len * sizeof(fe), &w));
+    STK_TRY(stk_stage(c, kSlotPolyB, coeff_bytes, {{0, coeffs.data(), coeff_bytes}}, &cf));
     STK_CUDA(c, cudaMemsetAsync(out, 0, nout * out_len * sizeof(fe), c->stream));
     return multivar_products(c, (const fe*)d_polys, h_lens, in_stride, width, h_mono_out, (const fe*)cf, h_mono_exps,
                              order, out, out_len, (fe*)w);
@@ -560,18 +553,18 @@ extern "C" __attribute__((visibility("default"))) int stk_poly_eval_multivar(
     for (uint64_t k = 0; k < 12; ++k) hm[t].exp[k] = k < width ? h_mono_exps[m * width + k] : 0;
   }
   const uint64_t stage_bytes = width * ms * sizeof(fe), mono_bytes = hm.size() * sizeof(PolyMonomial);
+  const uint64_t first_bytes = first.size() * sizeof(uint32_t);
   void* s1;
   void* s2;
-  STK_TRY(stk_scratch(c, kSlotComp, (width + nout) * L * sizeof(fe), &s1));
-  STK_TRY(stk_scratch(c, kSlotComp2, stage_bytes + mono_bytes + first.size() * sizeof(uint32_t), &s2));
+  STK_TRY(stk_scratch(c, kSlotPolyA, (width + nout) * L * sizeof(fe), &s1));
+  STK_TRY(stk_stage(c, kSlotPolyB, stage_bytes + mono_bytes + first_bytes,
+                    {{stage_bytes, hm.data(), mono_bytes}, {stage_bytes + mono_bytes, first.data(), first_bytes}},
+                    &s2));
   fe* Av = (fe*)s1;
   fe* E = Av + width * L;
   fe* stage = (fe*)s2;
-  PolyMonomial* d_monos = (PolyMonomial*)((char*)s2 + stage_bytes);
-  uint32_t* d_first = (uint32_t*)((char*)s2 + stage_bytes + mono_bytes);
-  STK_CUDA(c, cudaMemcpyAsync(d_monos, hm.data(), mono_bytes, cudaMemcpyHostToDevice, c->stream));
-  STK_CUDA(c, cudaMemcpyAsync(d_first, first.data(), first.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
-  STK_CUDA(c, cudaStreamSynchronize(c->stream));  // hm and first are stack-owned staging buffers
+  const PolyMonomial* d_monos = (const PolyMonomial*)((char*)s2 + stage_bytes);
+  const uint32_t* d_first = (const uint32_t*)((char*)s2 + stage_bytes + mono_bytes);
   STK_CUDA(c, cudaMemsetAsync(stage, 0, stage_bytes, c->stream));
   for (uint64_t k = 0; k < width; ++k) {
     const uint64_t nk = std::min(h_lens[k], ms);
@@ -580,13 +573,10 @@ extern "C" __attribute__((visibility("default"))) int stk_poly_eval_multivar(
                                   cudaMemcpyDeviceToDevice, c->stream));
   }
   STK_TRY(ntt_cols(c, stage, ms, ms, Av, L, width, R.w[s], 0));
-  if (c->is_stark)
-    multivar_eval_kernel<StarkField><<<blocks_for(L, 128), 128, 0, c->stream>>>(Av, L, (uint32_t)width, d_monos, d_first,
-                                                                                (uint32_t)nout, E, StarkField());
-  else
-    multivar_eval_kernel<MontField><<<blocks_for(L, 128), 128, 0, c->stream>>>(Av, L, (uint32_t)width, d_monos, d_first,
-                                                                               (uint32_t)nout, E, c->mont);
-  STK_CUDA(c, cudaGetLastError());
+  STK_TRY(stk_with_field(c, [&](auto f) {
+    multivar_eval_kernel<<<blocks_for(L, 128), 128, 0, c->stream>>>(Av, L, (uint32_t)width, d_monos, d_first,
+                                                                    (uint32_t)nout, E, f);
+  }));
   STK_TRY(ntt_cols(c, E, L, L, E, L, nout, R.w[s], 1));
   for (uint64_t j = 0; j < nout; ++j)
     STK_CUDA(c, cudaMemcpyAsync(out + j * out_len, E + j * L, out_len * sizeof(fe), cudaMemcpyDeviceToDevice, c->stream));

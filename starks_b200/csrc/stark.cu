@@ -23,8 +23,23 @@ struct Monomial {
   uint8_t exp[12];   // exponent of each state variable (width <= 12)
 };
 
-// One thread per evaluation point.  State values P_k(x_i) are loaded once; every monomial is
+// step_j(P_1(x_i), ..., P_w(x_i)) from the state in twiddle form: every monomial of output j is
 // coeff * prod_k P_k^e_k by repeated multiplication (degrees are tiny: <= extension factor).
+template <class F>
+__device__ __forceinline__ fe step_poly(const Monomial* __restrict__ monos, uint32_t nmono, uint32_t width, uint32_t j,
+                                        const fe* st_tw, const F& f) {
+  fe acc = fe_zero();
+  for (uint32_t m = 0; m < nmono; ++m) {
+    if (monos[m].out != j) continue;
+    fe term = f.from_tw(monos[m].coeff_tw);  // plain coefficient
+    for (uint32_t k = 0; k < width; ++k)
+      for (uint32_t e = 0; e < monos[m].exp[k]; ++e) term = f.mul_tw(term, st_tw[k]);
+    acc = f.add(acc, term);
+  }
+  return acc;
+}
+
+// One thread per evaluation point; the state values P_k(x_i) are loaded once.
 template <class F>
 __global__ void __launch_bounds__(128) constraint_eval_kernel(const fe* __restrict__ pev, uint64_t n, uint64_t ext,
                                                               uint32_t width, uint64_t col_stride,
@@ -39,14 +54,7 @@ __global__ void __launch_bounds__(128) constraint_eval_kernel(const fe* __restri
   }
   const uint64_t inext = (i + ext) % n;
   for (uint32_t j = 0; j < width; ++j) {
-    fe acc = fe_zero();
-    for (uint32_t m = 0; m < nmono; ++m) {
-      if (monos[m].out != j) continue;
-      fe term = f.from_tw(monos[m].coeff_tw);  // plain coefficient
-      for (uint32_t k = 0; k < width; ++k)
-        for (uint32_t e = 0; e < monos[m].exp[k]; ++e) term = f.mul_tw(term, st_tw[k]);
-      acc = f.add(acc, term);
-    }
+    const fe acc = step_poly(monos, nmono, width, j, st_tw, f);
     fe nxt = fe_load(pev + j * col_stride + inext);
     fe_store(cev + j * out_stride + i, f.sub(nxt, acc));
   }
@@ -82,14 +90,7 @@ __global__ void __launch_bounds__(128) quotient_eval_kernel(const fe* __restrict
   const fe xm = f.sub(fe_load_ro(X + (i << xshift)), last_tw);
   const fe fac_tw = f.to_tw(f.mul_tw(inv.v[r], xm));
   for (uint32_t j = 0; j < width; ++j) {
-    fe acc = fe_zero();
-    for (uint32_t m = 0; m < nmono; ++m) {
-      if (monos[m].out != j) continue;
-      fe term = f.from_tw(monos[m].coeff_tw);
-      for (uint32_t k = 0; k < width; ++k)
-        for (uint32_t e = 0; e < monos[m].exp[k]; ++e) term = f.mul_tw(term, st_tw[k]);
-      acc = f.add(acc, term);
-    }
+    const fe acc = step_poly(monos, nmono, width, j, st_tw, f);
     const fe cval = f.sub(fe_load(pev + j * col_stride + inext), acc);
     fe_store(dev + j * out_stride + i, f.mul_tw(cval, fac_tw));
   }
@@ -297,55 +298,39 @@ __global__ void __launch_bounds__(256) lincomb_kernel(const fe* __restrict__ col
   fe_store(out + i, acc);
 }
 
-template <class F>
-int div_linear_impl(stk_ctx* c, const fe* a, uint64_t n, const fe* rpow, uint64_t rs, const fe* rinvpow, uint64_t ris,
-                    fe* out, const F& f) {
-  const uint64_t per_block = (uint64_t)kScanChunk * kScanThreads;
-  const uint64_t nblocks = (n + per_block - 1) / per_block;
-  void* t;
-  STK_TRY(stk_scratch(c, 2, nblocks * sizeof(fe), &t));
-  fe* totals = (fe*)t;
-  scan_block_totals_kernel<F><<<(unsigned)nblocks, kScanThreads, 0, c->stream>>>(a, rpow, rs, n, totals, f);
-  scan_totals_kernel<F><<<1, kScanThreads, 0, c->stream>>>(totals, nblocks, f);
-  scan_finish_kernel<F><<<(unsigned)nblocks, kScanThreads, 0, c->stream>>>(a, rpow, rs, rinvpow, ris, n, totals, out, f);
-  STK_CUDA(c, cudaGetLastError());
+// The monomial list of the step polynomials: for monomial m, out[m] = constraint index,
+// coeffs[8*m..] = coefficient limbs (canonical), exps[width*m + k] = exponent of X_{k+1}.
+int pack_monomials(stk_ctx* c, uint64_t width, const uint32_t* h_mono_out, const uint32_t* h_mono_coeffs,
+                   const uint8_t* h_mono_exps, uint64_t nmono, std::vector<Monomial>& ms) {
+  ms.resize(nmono ? nmono : 1);
+  for (uint64_t m = 0; m < nmono; ++m) {
+    if (h_mono_out[m] >= width) return stk_fail(c, STK_EINVAL, "monomial output index out of range");
+    ms[m].coeff_tw = stk_h_to_tw(c, host::reduce(stk_load_fe(h_mono_coeffs + 8 * m), c->p));
+    ms[m].out = h_mono_out[m];
+    for (uint64_t k = 0; k < 12; ++k) ms[m].exp[k] = k < width ? h_mono_exps[width * m + k] : 0;
+  }
   return STK_OK;
 }
 
 }  // namespace
 
-#define STK_API extern "C" __attribute__((visibility("default")))
-
-// step polynomials as a monomial list: for monomial m, out[m] = constraint index,
-// coeffs[8*m..] = coefficient limbs (canonical), exps[width*m + k] = exponent of X_{k+1}.
+// step polynomials as a monomial list (pack_monomials)
 STK_API int stk_constraint_eval(stk_ctx* c, const uint32_t* d_pev, uint64_t n, uint64_t ext, uint64_t width,
                                 uint64_t col_stride, const uint32_t* h_mono_out, const uint32_t* h_mono_coeffs,
                                 const uint8_t* h_mono_exps, uint64_t nmono, uint32_t* d_cev, uint64_t out_stride) {
   if (!c || !d_pev || !d_cev || (!nmono ? false : (!h_mono_out || !h_mono_coeffs || !h_mono_exps))) return STK_EINVAL;
   if (width == 0 || width > 12) return stk_fail(c, STK_EUNSUPPORTED, "state width must be in 1..12");
-  std::vector<Monomial> ms(nmono ? nmono : 1);
-  for (uint64_t m = 0; m < nmono; ++m) {
-    if (h_mono_out[m] >= width) return stk_fail(c, STK_EINVAL, "monomial output index out of range");
-    fe cf = host::reduce(stk_load_fe(h_mono_coeffs + 8 * m), c->p);
-    ms[m].coeff_tw = stk_h_to_tw(c, cf);
-    ms[m].out = h_mono_out[m];
-    for (uint64_t k = 0; k < 12; ++k) ms[m].exp[k] = k < width ? h_mono_exps[width * m + k] : 0;
-  }
+  std::vector<Monomial> ms;
+  STK_TRY(pack_monomials(c, width, h_mono_out, h_mono_coeffs, h_mono_exps, nmono, ms));
+  const uint64_t mono_bytes = ms.size() * sizeof(Monomial);
   void* t;
-  STK_TRY(stk_scratch(c, 2, ms.size() * sizeof(Monomial), &t));
-  STK_CUDA(c, cudaMemcpyAsync(t, ms.data(), ms.size() * sizeof(Monomial), cudaMemcpyHostToDevice, c->stream));
-  STK_CUDA(c, cudaStreamSynchronize(c->stream));  // ms is a stack-owned staging buffer
+  STK_TRY(stk_stage(c, kSlotStage, mono_bytes, {{0, ms.data(), mono_bytes}}, &t));
   unsigned blocks = (unsigned)((n + 127) / 128);
-  if (c->is_stark)
-    constraint_eval_kernel<StarkField><<<blocks, 128, 0, c->stream>>>((const fe*)d_pev, n, ext, (uint32_t)width, col_stride,
-                                                                      (const Monomial*)t, (uint32_t)nmono, (fe*)d_cev,
-                                                                      out_stride, StarkField());
-  else
-    constraint_eval_kernel<MontField><<<blocks, 128, 0, c->stream>>>((const fe*)d_pev, n, ext, (uint32_t)width, col_stride,
-                                                                     (const Monomial*)t, (uint32_t)nmono, (fe*)d_cev,
-                                                                     out_stride, c->mont);
-  STK_CUDA(c, cudaGetLastError());
-  return STK_OK;
+  return stk_with_field(c, [&](auto f) {
+    constraint_eval_kernel<<<blocks, 128, 0, c->stream>>>((const fe*)d_pev, n, ext, (uint32_t)width, col_stride,
+                                                          (const Monomial*)t, (uint32_t)nmono, (fe*)d_cev, out_stride,
+                                                          f);
+  });
 }
 
 // construct_remainder_polynomials (stark.py:57-78) in evaluation form on the size-n domain <g2>:
@@ -363,16 +348,10 @@ STK_API int stk_quotient_eval(stk_ctx* c, const uint32_t* d_pev, uint64_t n, uin
   if (ext < 2 || ext > 16 || n % ext) return stk_fail(c, STK_EUNSUPPORTED, "extension factor must be in 2..16 and divide n");
   const uint64_t steps = n / ext;
   if (sub_n == 0 || sub_n % steps) return stk_fail(c, STK_EINVAL, "d_dsub must cover a subgroup containing <g2^ext>");
-  std::vector<Monomial> ms(nmono ? nmono : 1);
-  for (uint64_t m = 0; m < nmono; ++m) {
-    if (h_mono_out[m] >= width) return stk_fail(c, STK_EINVAL, "monomial output index out of range");
-    fe cf = host::reduce(stk_load_fe(h_mono_coeffs + 8 * m), c->p);
-    ms[m].coeff_tw = stk_h_to_tw(c, cf);
-    ms[m].out = h_mono_out[m];
-    for (uint64_t k = 0; k < 12; ++k) ms[m].exp[k] = k < width ? h_mono_exps[width * m + k] : 0;
-  }
+  std::vector<Monomial> ms;
+  STK_TRY(pack_monomials(c, width, h_mono_out, h_mono_coeffs, h_mono_exps, nmono, ms));
   const fe G2 = host::reduce(stk_load_fe(g2), c->p);
-  const fe one = host::reduce(host::from_u64(1), c->p);
+  const fe one = stk_h_one(c);
   if (!fe_eq(stk_h_pow(c, G2, n), one)) return stk_fail(c, STK_EINVAL, "g2^n != 1");
   const fe omega = stk_h_pow(c, G2, steps);
   QuotInv inv;
@@ -385,29 +364,19 @@ STK_API int stk_quotient_eval(stk_ctx* c, const uint32_t* d_pev, uint64_t n, uin
     wr = stk_h_mul(c, wr, omega);
   }
   const fe* X;
-  uint64_t xs = 1;
-  STK_TRY(stk_get_table_strided(c, G2, n, &X, &xs));
-  int xshift = 0;
-  while ((1ull << xshift) < xs) ++xshift;
-  if ((1ull << xshift) != xs) { STK_TRY(stk_get_table(c, G2, n, &X)); xshift = 0; }
+  int xshift;
+  STK_TRY(stk_get_table_shift(c, G2, n, &X, &xshift));
+  const uint64_t mono_bytes = ms.size() * sizeof(Monomial);
   void* t;
-  STK_TRY(stk_scratch(c, 2, ms.size() * sizeof(Monomial), &t));
-  STK_CUDA(c, cudaMemcpyAsync(t, ms.data(), ms.size() * sizeof(Monomial), cudaMemcpyHostToDevice, c->stream));
-  STK_CUDA(c, cudaStreamSynchronize(c->stream));  // ms is a stack-owned staging buffer
+  STK_TRY(stk_stage(c, kSlotStage, mono_bytes, {{0, ms.data(), mono_bytes}}, &t));
   const fe last_tw = stk_h_to_tw(c, host::reduce(stk_load_fe(last), c->p));
   unsigned blocks = (unsigned)((n + 127) / 128);
-  if (c->is_stark)
-    quotient_eval_kernel<StarkField><<<blocks, 128, 0, c->stream>>>((const fe*)d_pev, n, ext, (uint32_t)width, col_stride,
-                                                                    (const Monomial*)t, (uint32_t)nmono, X, xshift, last_tw, inv,
-                                                                    (const fe*)d_dsub, dsub_stride, sub_n / steps, (fe*)d_dev,
-                                                                    out_stride, StarkField());
-  else
-    quotient_eval_kernel<MontField><<<blocks, 128, 0, c->stream>>>((const fe*)d_pev, n, ext, (uint32_t)width, col_stride,
-                                                                   (const Monomial*)t, (uint32_t)nmono, X, xshift, last_tw, inv,
-                                                                   (const fe*)d_dsub, dsub_stride, sub_n / steps, (fe*)d_dev,
-                                                                   out_stride, c->mont);
-  STK_CUDA(c, cudaGetLastError());
-  return STK_OK;
+  return stk_with_field(c, [&](auto f) {
+    quotient_eval_kernel<<<blocks, 128, 0, c->stream>>>((const fe*)d_pev, n, ext, (uint32_t)width, col_stride,
+                                                        (const Monomial*)t, (uint32_t)nmono, X, xshift, last_tw, inv,
+                                                        (const fe*)d_dsub, dsub_stride, sub_n / steps, (fe*)d_dev,
+                                                        out_stride, f);
+  });
 }
 
 // construct_boundary_polynomials (stark.py:80-104) in evaluation form on the size-n domain <g2>
@@ -427,15 +396,10 @@ STK_API int stk_boundary_eval(stk_ctx* c, const uint32_t* d_pev, uint64_t n, uin
   if (ext < 2 || n % ext || last_index % ext || last_index >= n || last_index == 0)
     return stk_fail(c, STK_EINVAL, "last_index must be a non-zero multiple of ext below n");
   const fe G2 = host::reduce(stk_load_fe(g2), c->p);
-  const fe one = host::reduce(host::from_u64(1), c->p);
-  if (!fe_eq(stk_h_pow(c, G2, n), one) || fe_eq(stk_h_pow(c, G2, n / 2), one))
-    return stk_fail(c, STK_EINVAL, "g2 is not a primitive n-th root of unity");
+  if (!stk_h_primitive(c, G2, n)) return stk_fail(c, STK_EINVAL, "g2 is not a primitive n-th root of unity");
   const fe* X;
-  uint64_t xs = 1;
-  STK_TRY(stk_get_table_strided(c, G2, n, &X, &xs));
-  int xshift = 0;
-  while ((1ull << xshift) < xs) ++xshift;
-  if ((1ull << xshift) != xs) { STK_TRY(stk_get_table(c, G2, n, &X)); xshift = 0; }
+  int xshift;
+  STK_TRY(stk_get_table_shift(c, G2, n, &X, &xshift));
   // per-context cache (least recently used first), bounded by kInvTableCacheBytes; only this
   // context's own stream can still be reading an evicted table, and it is synchronised first
   fe* T = nullptr;
@@ -482,17 +446,14 @@ STK_API int stk_quotient_z(stk_ctx* c, const uint32_t* d_ccoef, uint64_t n, uint
                            uint32_t* d_dcoef, uint32_t* h_bad) {
   if (!c || !d_ccoef || !d_dcoef || !last || steps == 0 || n % steps) return STK_EINVAL;
   void* t;
-  STK_TRY(stk_scratch(c, 2, 64, &t));
+  STK_TRY(stk_scratch(c, kSlotStage, 64, &t));
   STK_CUDA(c, cudaMemsetAsync(t, 0, 4, c->stream));
   fe last_tw = stk_h_to_tw(c, host::reduce(stk_load_fe(last), c->p));
   unsigned blocks = (unsigned)((steps + 255) / 256);
-  if (c->is_stark)
-    quotient_z_kernel<StarkField><<<blocks, 256, 0, c->stream>>>((const fe*)d_ccoef, n, steps, last_tw, (fe*)d_dcoef,
-                                                                 (uint32_t*)t, StarkField());
-  else
-    quotient_z_kernel<MontField><<<blocks, 256, 0, c->stream>>>((const fe*)d_ccoef, n, steps, last_tw, (fe*)d_dcoef,
-                                                                (uint32_t*)t, c->mont);
-  STK_CUDA(c, cudaGetLastError());
+  STK_TRY(stk_with_field(c, [&](auto f) {
+    quotient_z_kernel<<<blocks, 256, 0, c->stream>>>((const fe*)d_ccoef, n, steps, last_tw, (fe*)d_dcoef, (uint32_t*)t,
+                                                     f);
+  }));
   if (h_bad) {
     STK_CUDA(c, cudaMemcpyAsync(h_bad, t, 4, cudaMemcpyDeviceToHost, c->stream));
     STK_CUDA(c, cudaStreamSynchronize(c->stream));
@@ -507,7 +468,7 @@ STK_API int stk_div_linear(stk_ctx* c, const uint32_t* d_a, uint64_t n, const ui
                            uint32_t* d_out) {
   if (!c || !d_a || !d_out || !r || n < 2) return STK_EINVAL;
   fe rr = host::reduce(stk_load_fe(r), c->p);
-  fe one = host::reduce(host::from_u64(1), c->p);
+  fe one = stk_h_one(c);
   const fe* rpow = nullptr;
   const fe* rinvpow = nullptr;
   uint64_t rs = 1, ris = 1;
@@ -517,8 +478,18 @@ STK_API int stk_div_linear(stk_ctx* c, const uint32_t* d_a, uint64_t n, const ui
     STK_TRY(stk_get_table_strided(c, rr, r_order, &rpow, &rs));
     STK_TRY(stk_get_table_strided(c, stk_h_inv(c, rr), r_order, &rinvpow, &ris));
   }
-  if (c->is_stark) return div_linear_impl<StarkField>(c, (const fe*)d_a, n, rpow, rs, rinvpow, ris, (fe*)d_out, StarkField());
-  return div_linear_impl<MontField>(c, (const fe*)d_a, n, rpow, rs, rinvpow, ris, (fe*)d_out, c->mont);
+  const fe* a = (const fe*)d_a;
+  fe* out = (fe*)d_out;
+  const uint64_t per_block = (uint64_t)kScanChunk * kScanThreads;
+  const uint64_t nblocks = (n + per_block - 1) / per_block;
+  void* t;
+  STK_TRY(stk_scratch(c, kSlotStage, nblocks * sizeof(fe), &t));
+  fe* totals = (fe*)t;
+  return stk_with_field(c, [&](auto f) {
+    scan_block_totals_kernel<<<(unsigned)nblocks, kScanThreads, 0, c->stream>>>(a, rpow, rs, n, totals, f);
+    scan_totals_kernel<<<1, kScanThreads, 0, c->stream>>>(totals, nblocks, f);
+    scan_finish_kernel<<<(unsigned)nblocks, kScanThreads, 0, c->stream>>>(a, rpow, rs, rinvpow, ris, n, totals, out, f);
+  });
 }
 
 // out[i] = sum_c weights[c] * cols[c][i]
@@ -528,75 +499,10 @@ STK_API int stk_lincomb(stk_ctx* c, const uint32_t* d_cols, uint64_t n, uint64_t
   std::vector<fe> w(ncols);
   for (uint64_t i = 0; i < ncols; ++i) w[i] = stk_h_to_tw(c, host::reduce(stk_load_fe(h_weights + 8 * i), c->p));
   void* t;
-  STK_TRY(stk_scratch(c, 2, ncols * sizeof(fe), &t));
-  STK_CUDA(c, cudaMemcpyAsync(t, w.data(), ncols * sizeof(fe), cudaMemcpyHostToDevice, c->stream));
-  STK_CUDA(c, cudaStreamSynchronize(c->stream));
+  STK_TRY(stk_stage(c, kSlotStage, ncols * sizeof(fe), {{0, w.data(), ncols * sizeof(fe)}}, &t));
   unsigned blocks = (unsigned)((n + 255) / 256);
-  if (c->is_stark)
-    lincomb_kernel<StarkField><<<blocks, 256, 0, c->stream>>>((const fe*)d_cols, n, (uint32_t)ncols, col_stride,
-                                                              (const fe*)t, (fe*)d_out, StarkField());
-  else
-    lincomb_kernel<MontField><<<blocks, 256, 0, c->stream>>>((const fe*)d_cols, n, (uint32_t)ncols, col_stride,
-                                                             (const fe*)t, (fe*)d_out, c->mont);
-  STK_CUDA(c, cudaGetLastError());
-  return STK_OK;
-}
-
-// get_computational_trace (starks/air.py:31-52) + the witness transposition of AIR.generate_witness
-// (:124): state[i+1][j] = step_poly_j(state[i]).  The recurrence is sequential by nature (one
-// 256-bit dependency chain of `steps` links), so it runs on one host core in the Montgomery
-// domain (hostmath.h) and writes witness[dim][step] in the ABI element layout -- pinned memory
-// from stk_host_alloc makes the following upload a single DMA.  Same monomial encoding as
-// stk_constraint_eval.
-STK_API int stk_trace_generate(stk_ctx* c, const uint32_t* h_inp, uint64_t steps, uint64_t width,
-                               const uint32_t* h_mono_out, const uint32_t* h_mono_coeffs, const uint8_t* h_mono_exps,
-                               uint64_t nmono, uint32_t* h_witness) {
-  if (!c || !h_inp || !h_witness || steps == 0 || (nmono && (!h_mono_out || !h_mono_coeffs || !h_mono_exps)))
-    return STK_EINVAL;
-  if (width == 0 || width > 12) return stk_fail(c, STK_EUNSUPPORTED, "state width must be in 1..12");
-  typedef unsigned __int128 u128;
-  const host::HostMont& H = host::host_mont(c->p);
-  struct M64 { uint64_t v[4]; };
-  auto addm = [&](const M64& a, const M64& b) {
-    M64 r;
-    u128 cy = 0;
-    for (int i = 0; i < 4; ++i) { cy += (u128)a.v[i] + b.v[i]; r.v[i] = (uint64_t)cy; cy >>= 64; }
-    bool ge = cy != 0;
-    if (!ge) {
-      ge = true;
-      for (int i = 3; i >= 0; --i) { if (r.v[i] > H.m[i]) break; if (r.v[i] < H.m[i]) { ge = false; break; } }
-    }
-    if (ge) {
-      uint64_t bw = 0;
-      for (int i = 0; i < 4; ++i) { u128 d = (u128)r.v[i] - H.m[i] - bw; r.v[i] = (uint64_t)d; bw = (uint64_t)(d >> 64) & 1; }
-    }
-    return r;
-  };
-  auto to_mont = [&](const fe& x) { M64 a, r; host::to64(x, a.v); host::mont64(H, a.v, H.r2, r.v); return r; };
-  const uint64_t one_plain[4] = {1, 0, 0, 0};
-  std::vector<M64> coef(nmono ? nmono : 1);
-  for (uint64_t m = 0; m < nmono; ++m) {
-    if (h_mono_out[m] >= width) return stk_fail(c, STK_EINVAL, "monomial output index out of range");
-    coef[m] = to_mont(host::reduce(stk_load_fe(h_mono_coeffs + 8 * m), c->p));
-  }
-  M64 st[12], nx[12];
-  for (uint64_t k = 0; k < width; ++k) st[k] = to_mont(host::reduce(stk_load_fe(h_inp + 8 * k), c->p));
-  for (uint64_t i = 0; i < steps; ++i) {
-    for (uint64_t k = 0; k < width; ++k) {  // leave the Montgomery domain on the way out
-      uint64_t plain[4];
-      host::mont64(H, st[k].v, one_plain, plain);
-      fe o = host::from64(plain);
-      memcpy(h_witness + (k * steps + i) * 8, o.v, 32);
-    }
-    if (i + 1 == steps) break;
-    for (uint64_t j = 0; j < width; ++j) memset(nx[j].v, 0, 32);
-    for (uint64_t m = 0; m < nmono; ++m) {
-      M64 t = coef[m];
-      for (uint64_t k = 0; k < width; ++k)
-        for (uint32_t e = 0; e < h_mono_exps[width * m + k]; ++e) host::mont64(H, t.v, st[k].v, t.v);
-      nx[h_mono_out[m]] = addm(nx[h_mono_out[m]], t);
-    }
-    for (uint64_t j = 0; j < width; ++j) st[j] = nx[j];
-  }
-  return STK_OK;
+  return stk_with_field(c, [&](auto f) {
+    lincomb_kernel<<<blocks, 256, 0, c->stream>>>((const fe*)d_cols, n, (uint32_t)ncols, col_stride, (const fe*)t,
+                                                  (fe*)d_out, f);
+  });
 }

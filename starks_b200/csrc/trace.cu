@@ -10,8 +10,8 @@
 //     walks the `steps/L` chunk starts with one matrix-vector product each (a prefix over powers
 //     of A: ~(w+1)^2 host multiplies per chunk), and the device runs every chunk's L links in
 //     its own thread.  Exact arithmetic: the trace is the sequential one bit for bit.
-//   * ONE trace of a non-linear AIR stays a single dependency chain: stk_trace_generate (host,
-//     stark.cu) or stk_trace_generate_upload below, which hides the host recurrence behind the
+//   * ONE trace of a non-linear AIR stays a single dependency chain: stk_trace_generate (host)
+//     or stk_trace_generate_upload below, which hides the host recurrence behind the
 //     upload of the blocks already generated.
 // Witness layout on the device: d_witness[(t*width + dim)*stride + step], ABI elements.
 #include <algorithm>
@@ -19,8 +19,6 @@
 #include "ctx.h"
 
 using namespace stk;
-
-#define STK_API extern "C" __attribute__((visibility("default")))
 
 namespace {
 
@@ -121,7 +119,7 @@ int pack_monomials(stk_ctx* c, uint64_t width, const uint32_t* h_mono_out, const
   monos.resize(nmono ? nmono : 1);
   memset(monos.data(), 0, monos.size() * sizeof(TraceMono));
   *linear = true;
-  const fe one = host::reduce(host::from_u64(1), c->p);
+  const fe one = stk_h_one(c);
   for (uint64_t m = 0; m < nmono; ++m) {
     if (h_mono_out[m] >= width) return stk_fail(c, STK_EINVAL, "monomial output index out of range");
     const fe co = host::reduce(stk_load_fe(h_mono_coeffs + 8 * m), c->p);
@@ -145,7 +143,7 @@ STK_API int stk_count_noncanonical(stk_ctx* c, const uint32_t* d_vals, uint64_t 
   *h_bad = 0;
   if (!n) return STK_OK;
   void* t;
-  STK_TRY(stk_scratch(c, 10, 64, &t));  // its own slot: the counter outlives this call when sync = 0
+  STK_TRY(stk_scratch(c, kSlotCounter, 64, &t));
   STK_CUDA(c, cudaMemsetAsync(t, 0, 4, c->stream));
   noncanonical_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>((const fe*)d_vals, n, c->p, (uint32_t*)t);
   STK_CUDA(c, cudaGetLastError());
@@ -229,22 +227,58 @@ STK_API int stk_trace_generate_dev(stk_ctx* c, const uint32_t* h_inp, uint64_t n
   }
   void* dm;
   const uint64_t mono_bytes = monos.size() * sizeof(TraceMono);
-  const uint64_t start_bytes = starts.size() * sizeof(fe);
-  STK_TRY(stk_scratch(c, 2, mono_bytes + start_bytes + 64, &dm));
-  fe* d_starts = (fe*)dm;
-  TraceMono* d_monos = (TraceMono*)((char*)dm + ((start_bytes + 63) / 64) * 64);
-  STK_CUDA(c, cudaMemcpyAsync(d_starts, starts.data(), start_bytes, cudaMemcpyHostToDevice, c->stream));
-  STK_CUDA(c, cudaMemcpyAsync(d_monos, monos.data(), mono_bytes, cudaMemcpyHostToDevice, c->stream));
-  STK_CUDA(c, cudaStreamSynchronize(c->stream));   // the staging vectors die with this frame
+  const uint64_t start_bytes = starts.size() * sizeof(fe), mono_off = ((start_bytes + 63) / 64) * 64;
+  STK_TRY(stk_stage(c, kSlotStage, mono_bytes + start_bytes + 64,
+                    {{0, starts.data(), start_bytes}, {mono_off, monos.data(), mono_bytes}}, &dm));
+  const fe* d_starts = (const fe*)dm;
+  const TraceMono* d_monos = (const TraceMono*)((char*)dm + mono_off);
   const unsigned blocks = (unsigned)((nthreads + 127) / 128);
-  if (c->is_stark)
-    trace_chunk_kernel<StarkField><<<blocks, 128, 0, c->stream>>>(d_starts, nthreads, nchunks, L, steps, (uint32_t)width,
-                                                                 d_monos, (uint32_t)nmono, (fe*)d_witness, stride,
-                                                                 StarkField());
-  else
-    trace_chunk_kernel<MontField><<<blocks, 128, 0, c->stream>>>(d_starts, nthreads, nchunks, L, steps, (uint32_t)width,
-                                                                d_monos, (uint32_t)nmono, (fe*)d_witness, stride, c->mont);
-  STK_CUDA(c, cudaGetLastError());
+  return stk_with_field(c, [&](auto f) {
+    trace_chunk_kernel<<<blocks, 128, 0, c->stream>>>(d_starts, nthreads, nchunks, L, steps, (uint32_t)width, d_monos,
+                                                      (uint32_t)nmono, (fe*)d_witness, stride, f);
+  });
+}
+
+// get_computational_trace (starks/air.py:31-52) + the witness transposition of AIR.generate_witness
+// (:124): state[i+1][j] = step_poly_j(state[i]).  The recurrence is sequential by nature (one
+// 256-bit dependency chain of `steps` links), so it runs on one host core in the Montgomery
+// domain (hostmath.h) and writes witness[dim][step] in the ABI element layout -- pinned memory
+// from stk_host_alloc makes the following upload a single DMA.  Same monomial encoding as
+// stk_trace_generate_dev.
+STK_API int stk_trace_generate(stk_ctx* c, const uint32_t* h_inp, uint64_t steps, uint64_t width,
+                               const uint32_t* h_mono_out, const uint32_t* h_mono_coeffs, const uint8_t* h_mono_exps,
+                               uint64_t nmono, uint32_t* h_witness) {
+  if (!c || !h_inp || !h_witness || steps == 0 || (nmono && (!h_mono_out || !h_mono_coeffs || !h_mono_exps)))
+    return STK_EINVAL;
+  if (width == 0 || width > 12) return stk_fail(c, STK_EUNSUPPORTED, "state width must be in 1..12");
+  const host::HostMont& H = host::host_mont(c->p);
+  struct M64 { uint64_t v[4]; };
+  auto to_mont = [&](const fe& x) { M64 a, r; host::to64(x, a.v); host::mont64(H, a.v, H.r2, r.v); return r; };
+  const uint64_t one_plain[4] = {1, 0, 0, 0};
+  std::vector<M64> coef(nmono ? nmono : 1);
+  for (uint64_t m = 0; m < nmono; ++m) {
+    if (h_mono_out[m] >= width) return stk_fail(c, STK_EINVAL, "monomial output index out of range");
+    coef[m] = to_mont(host::reduce(stk_load_fe(h_mono_coeffs + 8 * m), c->p));
+  }
+  M64 st[12], nx[12];
+  for (uint64_t k = 0; k < width; ++k) st[k] = to_mont(host::reduce(stk_load_fe(h_inp + 8 * k), c->p));
+  for (uint64_t i = 0; i < steps; ++i) {
+    for (uint64_t k = 0; k < width; ++k) {  // leave the Montgomery domain on the way out
+      uint64_t plain[4];
+      host::mont64(H, st[k].v, one_plain, plain);
+      fe o = host::from64(plain);
+      memcpy(h_witness + (k * steps + i) * 8, o.v, 32);
+    }
+    if (i + 1 == steps) break;
+    for (uint64_t j = 0; j < width; ++j) memset(nx[j].v, 0, 32);
+    for (uint64_t m = 0; m < nmono; ++m) {
+      M64 t = coef[m];
+      for (uint64_t k = 0; k < width; ++k)
+        for (uint32_t e = 0; e < h_mono_exps[width * m + k]; ++e) host::mont64(H, t.v, st[k].v, t.v);
+      add64m(H, nx[h_mono_out[m]].v, t.v, nx[h_mono_out[m]].v);
+    }
+    for (uint64_t j = 0; j < width; ++j) st[j] = nx[j];
+  }
   return STK_OK;
 }
 

@@ -11,7 +11,7 @@ unchanged."""
 import numpy as np
 import pytest
 
-from test_gpu_poly import BLS12_381_R, BN254_R, P, Guarded, full_range, limbs, padded, unchanged, upload
+from test_gpu_poly import BLS12_381_R, BN254_R, P, Guarded, full_range, ints, limbs, padded, unchanged, upload
 
 pytestmark = pytest.mark.gpu
 slow = pytest.mark.slow
@@ -304,6 +304,26 @@ def test_multivar_runtime_modulus(eng, oracle, name, p):
   sp = [{(0, 1): 1}, {(1, 0): 1, (0, 3): p - 2, (0, 0): 7}, {(2, 2): 1}]
   check_multivar(eng, oracle, p, [full_range(rng, 30, p), full_range(rng, 17, p)], sp)
   check_multivar(eng, oracle, p, [full_range(rng, 3, p)], [{(256,): 1}, {(300,): 2, (1,): 1}])
+
+
+def test_multivar_outputs_beyond_a_grid_dimension(eng):
+  """The batched inverse transform of multivariate evaluation has one column per output.  Over
+  BN254's scalar field a transform of length 2048 takes two passes, whose launches hold at most
+  65535 columns: 65 537 outputs (j + 1) x of a 1025-coefficient x must come back whole on both
+  sides of every column group."""
+  import torch
+  p, n, nout = BN254_R, 1025, 65537
+  x = full_range(np.random.default_rng(11), n, p)
+  eng.set_field(p)
+  dx = torch.from_numpy(limbs(x).view(np.int32)).cuda()
+  out = torch.empty((nout, n, 8), dtype=torch.int32, device="cuda")
+  torch.cuda.synchronize()
+  eng.poly_eval_multivar(dx.data_ptr(), [n], n, [(j, j + 1, (1,)) for j in range(nout)], nout, out.data_ptr(), n)
+  eng.sync()
+  for j in (0, 1, 32767, 32768, 65535, 65536):
+    assert ints(out[j].cpu().numpy().view(np.uint32)) == [(j + 1) * v % p for v in x], j
+  del dx, out
+  torch.cuda.empty_cache()
 
 
 # p = 31 has roots of order 2 only, p = 97 up to 32: the product / direct route, na > p included
